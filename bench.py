@@ -2,7 +2,7 @@
 """bench.py -- MCTS simulations/second of the batched sampled-MCTS hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 3m] [--mode joint|seq] [--impl ours|reference]
-                    [--total-roots T] [--legal-frac 0.7] [--no-extras]
+                    [--total-roots T] [--legal-frac 0.7] [--no-extras] [--dump-outputs DIR]
 
 A "step" is ONE whole search of the workload: B roots x S simulations (root preparation -> tree construction -> S x [select ->
 gather hidden -> recurrent_inference -> softmax/beta -> expand+backup] -> 13 readouts).  Default workload is BASELINE.json
@@ -22,6 +22,12 @@ states and random-init weights of the reference architecture.
 `--impl reference` times the reference's CPU path alone (the reference arm).
 N > 1: roots sharded by rank (weak scaling by default, `--total-roots` = strong scaling), ONE all-gather of the packed readouts per
 search (`SampledMCTS.batch_search_sharded` is the product entry; the device-resident step issues the same collective).
+`--dump-outputs DIR` writes the readouts of the last timed device-resident search (rank 0's roots) as DIR/<name>.npy: the inputs
+depend only on the arguments, so two builds can be compared output for output.
+
+libmaz_b200.so is rebuilt only when it is missing or older than its sources, and the CPU checker (oracle/) is loaded as built,
+compiled only when missing: on a tree that `__graft_entry__.build()` has built, the benchmark compiles and writes nothing, so
+that tree may be read-only.
 """
 import argparse
 import json
@@ -68,7 +74,34 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the sequential-mode / legal-mask / other-config legs")
     ap.add_argument("--inference", default="bf16", choices=["bf16", "fp32"], help="bf16 = fused kernels, fp32 = parity mode")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the readouts of the last timed search as DIR/<name>.npy (float32, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, out, limit=DUMP_LIMIT):
+    """Write the readouts of one search (`out`: name -> device tensor with the roots along dim 0) as path/<name>.npy in float32
+    (the integer readouts -- counts, actions -- are exact in float32).  When all roots would take more than `limit` bytes, a fixed
+    sample of roots (seed 0, in root order) is written, and its root indices as root_index.npy (float64)."""
+    arrs = {k: v.cpu().numpy().astype(np.float32) for k, v in out.items()}
+    B = len(arrs["value"])
+    hdr = 128 * (len(arrs) + 1)                                    # one .npy header per file
+    per_root = sum(a[0].nbytes for a in arrs.values())
+    if B * per_root + hdr > limit:
+        keep = np.sort(np.random.RandomState(0).choice(B, (limit - hdr) // (per_root + 8), replace=False))
+        arrs = {k: a[keep] for k, a in arrs.items()}
+        arrs["root_index"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def workload(args, world=1):
@@ -171,7 +204,6 @@ def cpu_reference_search(args, N, A, B, S, K, sd, hidden, steps, warmup, device=
     from oracle.model_oracle import inverse_support_transform
     from oracle.search_oracle import NetworkOutput, reference_batch_search
 
-    pyoracle.build()
     kind = "reference" if pyoracle.available("reference") else "port"
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
@@ -208,7 +240,6 @@ def cpu_ctree_only(N, A, B, S, K, joint, steps=2, warmup=1):
     from _harness import MCTS, Inputs, drive
     from oracle import pyoracle
 
-    pyoracle.build()
     kind = "reference" if pyoracle.available("reference") else "port"
     Nt = N if joint else 1
     inp = Inputs(B, Nt, A, S, seed=0, mode="random")
@@ -428,6 +459,8 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     ex = Exchange(True)
     ms_dev = timed(make_dev_step(ex), steps, warm)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, plan.out)        # before any further search overwrites the readouts
     # a default run times 10 short searches: shorter than nvidia-smi's start-up.  Keep the GPU under the same load (untimed
     # steps, the same number on every rank) until ~0.4 s have passed, so that the clocks are sampled under load.
     extra = int(max(0.0, 0.4 - steps * ms_dev * 1e-3) / (ms_dev * 1e-3)) + 1

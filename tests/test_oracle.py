@@ -22,6 +22,7 @@ class GoldenInputs:
                          lam=float(m[4]), delta_lb=float(m[5]))
         self.seed = int(z["tree_seed"])
         self.expected = {k[4:]: z[k] for k in z.files if k.startswith("out_")}
+        self.tot_nodes = z["tot_nodes"]
 
 
 def check_golden(make_tree, path, exact=True):
@@ -38,6 +39,7 @@ def check_golden(make_tree, path, exact=True):
                                   b.view(np.int32) if b.dtype == np.float32 else b), f"{os.path.basename(path)}:{k}"
         else:
             np.testing.assert_allclose(a, b, rtol=1e-5, atol=1e-7, err_msg=k)
+    assert np.array_equal(tree.stats()[0], g.tot_nodes), f"{os.path.basename(path)}: node counts"
     return tree
 
 

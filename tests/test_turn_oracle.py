@@ -31,6 +31,26 @@ def test_eps_greedy_reproduces_reference_known_answers():
         assert eps_greedy_action(z["greedy"][i], float(z["eps"]), z["eps_u"][i], z["rand_act"][i]) == z["eps_result"][i]
 
 
+def test_turn_draws_from_seeds_reproduce_reference_known_answers():
+    """The draws of the live comparison below, made here from the seeds the known answers were recorded with:
+    np.random.RandomState(1000 + i) for select_action; for eps_greedy_action torch.manual_seed(i), then one rand_like draw,
+    then Categorical(mask).sample(), the order in which the reference consumes torch's global generator."""
+    from oracle.turn_oracle import eps_greedy_action, select_action
+
+    z = np.load(KAT)
+    for i in range(len(z["lens"])):
+        c = z["counts"][i, : z["lens"][i]]
+        u = np.random.RandomState(1000 + i).random_sample()
+        pos, ent = select_action(c, temperature=float(z["temps"][i]), deterministic=False, uniform=u)
+        assert pos == z["pos"][i] and ent == z["entropy"][i], i
+    for i in range(len(z["greedy"])):
+        torch.manual_seed(i)
+        m = torch.from_numpy(z["masks"][i])
+        u = float(torch.rand_like(m[..., 0].float()))
+        ra = int(torch.distributions.Categorical(m).sample())
+        assert eps_greedy_action(int(z["greedy"][i]), float(z["eps"]), u, ra) == z["eps_result"][i], i
+
+
 @pytest.mark.skipif(not os.path.exists(os.path.join(REF, "core", "utils.py")), reason="reference sources not present on this box")
 def test_turn_functions_equal_reference_live():
     import sys
