@@ -97,6 +97,13 @@ def _output_from_readout(r):
                         rg("mcts_values"), rg("rewards"), rg("qvalues"))
 
 
+def _local_agent_turns(plan, count):
+    """The first `count` roots of a sequential-agent plan's step results (one D2H copy, one sync): a rank's own slice."""
+    outs, actions, dist, prob, entropy = plan.finish_turns()
+    return AgentTurnsOutput(actions[:count], dist[:count], prob[:count], entropy[:count],
+                            [_output_from_readout({k: v[:count] for k, v in r.items()}) for r in outs])
+
+
 class _DevicePlan:
     """Static buffers + the captured CUDA graphs of S simulations for one problem shape.  The sequential-agent turns
     (current_agent_idx = 0..N-1) share ONE plan -- tree arena, hidden-state pool and staging buffers are by far the
@@ -166,7 +173,7 @@ class _DevicePlan:
         out_spec = [(f"t{t}", i32, (words,)) for t in range(T)]
         out_spec += [("turn_actions", i32, (B, self.N)), ("prob_prod", f64, (B,)),
                      ("policy_dist", f64, (B, self.N, self.A)), ("entropy", f64, (B, self.N))]
-        self.res, self.res_np, self.res_flat, self.res_host, _ = self._flat(out_spec, dev)
+        self.res, self.res_np, self.res_flat, self.res_host, self.res_off = self._flat(out_spec, dev)
         self.words = words
         self.turn_out, self.turn_out_np = [], []
         for t in range(T):
@@ -194,6 +201,24 @@ class _DevicePlan:
             g = (dev, torch.empty(dev.numel(), dtype=torch.int32).pin_memory())
             self._gather = g
         return g
+
+    def turn_gather_buffers(self, world):
+        """(device, pinned host) int32 buffers for the all-gather of `world` whole step buffers (`res_flat`: every agent's
+        readouts + the turn results)."""
+        g = getattr(self, "_turn_gather", None)
+        if g is None or g[0].numel() != world * self.res_flat.numel():
+            dev = torch.empty(world * self.res_flat.numel(), dtype=torch.int32, device=self.dev)
+            g = (dev, torch.empty(dev.numel(), dtype=torch.int32).pin_memory())
+            self._turn_gather = g
+        return g
+
+    def turn_layout(self):
+        """Where everything lives in `res_flat` (int32 words): (readout_spec, word offset of each turn's readout block,
+        [(name, numpy dtype, shape, word offset)] of the turn fields) -- what `sharding.split_turn_block` reads."""
+        npdt = {torch.float32: np.float32, torch.int32: np.int32, torch.float64: np.float64}
+        fields = [(n, npdt[self.res[n].dtype], tuple(self.res[n].shape), self.res_off[n][0])
+                  for n in ("turn_actions", "prob_prod", "policy_dist", "entropy")]
+        return self.readout_spec, [self.res_off[f"t{t}"][0] for t in range(self.T)], fields
 
     def device_bytes(self):
         """HBM held by this plan (pool + arena + loop buffers + staging mirrors)."""
@@ -804,6 +829,79 @@ class SampledMCTS(object):
                               root_index_offset)
         outs, actions, dist, prob, entropy = plan.finish_turns()
         return AgentTurnsOutput(actions, dist, prob, entropy, [_output_from_readout(r) for r in outs])
+
+    # ---- SURVEY 8(e) + 8(f): the per-agent loop of one environment step with the roots sharded over the ranks, ONE exchange ------
+    def search_agents_sharded(self, model, network_output, true_num_agents: int, total_roots: int, legal_actions_lst=None,
+                              device=None, add_noise: bool = True, sampled_tau: float = 1.0, turn: str = "greedy",
+                              temperature: float = 1.0, greedy_epsilon: float = 0.0, eps_randoms=None, group=None,
+                              gather: bool = True) -> AgentTurnsOutput:
+        """`search_agents` for a batch of `total_roots` roots split over the ranks of `group` (torch.distributed, NCCL).  This rank
+        passes ITS contiguous slice `sharding.shard_range(total_roots, rank, world)` of every per-root argument (`network_output`,
+        `legal_actions_lst`, and each (N, count) array of `eps_randoms`) and runs all N turns on it with no exchange: agent k+1's
+        `factor` for a root depends only on that root's own trees.  After the last turn ONE all-gather of the whole step buffer
+        (every agent's readouts + the turn results) gives every rank the AgentTurnsOutput of all roots in global order.
+        Every rank must hold `np_random` in the same state: each draws what single-process `search_agents` over `total_roots`
+        roots would draw and keeps its slice, so the result and the final generator state do not depend on the number of ranks.
+        gather=False returns the local slice only (no collective)."""
+        import torch.distributed as dist
+
+        from . import sharding
+
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+        plan, count = self._search_agents_rank(model, network_output, true_num_agents, total_roots, rank, world, legal_actions_lst,
+                                               device, add_noise, sampled_tau, turn, temperature, greedy_epsilon, eps_randoms)
+        if not gather or world == 1:
+            return _local_agent_turns(plan, count)
+        gbuf, ghost = plan.turn_gather_buffers(world)
+        dist.all_gather_into_tensor(gbuf, plan.res_flat, group=group)              # the one collective of the environment step
+        ghost.copy_(gbuf, non_blocking=True)
+        plan.tree.check()
+        outs, t = sharding.merge_turn_shards(ghost.numpy().reshape(world, -1), plan.turn_layout(), total_roots, world)
+        return AgentTurnsOutput(t["turn_actions"], t["policy_dist"], t["prob_prod"], t["entropy"], [_output_from_readout(r) for r in outs])
+
+    def _search_agents_rank(self, model, network_output, true_num_agents, total_roots, rank, world, legal_actions_lst=None,
+                            device=None, add_noise=True, sampled_tau=1.0, turn="greedy", temperature=1.0, greedy_epsilon=0.0,
+                            eps_randoms=None):
+        """The body of `search_agents_sharded` on rank `rank` of `world`, with no collective and no host sync: the N turns of
+        this rank's slice, padded to the largest shard, are enqueued on the plan's stream.  Returns (plan, local root count);
+        the step's results land in `plan.res_flat`."""
+        from . import sharding
+
+        cfg = self.config
+        N, A = int(true_num_agents), cfg.action_space_size
+        inf = self._device_inference(model, device)
+        if inf is None:
+            raise RuntimeError("search_agents_sharded needs a network with a device path (SMAC / matrix MAMuZeroNet on a CUDA device)")
+        if turn not in ("greedy", "sample"):
+            raise ValueError(turn)
+        start, count = sharding.shard_range(total_roots, rank, world)
+        Bp = sharding.shard_range(total_roots, 0, world)[1]               # the largest shard: every rank searches Bp roots
+        if count == 0:
+            raise ValueError(f"{total_roots} roots cannot be split over {world} ranks")
+        eps_u, rand_act = (None, None) if eps_randoms is None else eps_randoms
+        for x in (network_output.hidden_state, legal_actions_lst):
+            if x is not None and x.shape[0] != count:
+                raise ValueError(f"rank {rank}: expected {count} local roots, got {x.shape[0]}")
+        for x in (eps_u, rand_act):
+            if x is not None and tuple(np.shape(x)) != (N, count):
+                raise ValueError(f"rank {rank}: expected {count} local roots, got eps_randoms of shape {tuple(np.shape(x))}")
+        pad = lambda x: None if x is None else sharding.pad_rows(x, Bp)
+        noise_epsilon = cfg.root_exploration_fraction if add_noise else 0.0
+        plan = self._plan(inf, Bp, 0, sampled_tau)
+        plan.stage_roots(pad(network_output.hidden_state), pad(network_output.reward), pad(network_output.value),
+                         pad(network_output.policy_logits), pad(legal_actions_lst))
+        plan.begin_turns()
+        mine = slice(start, start + count)
+        for k in range(N):       # np_random is consumed as single-process search_agents over total_roots roots consumes it
+            noises = hostrng.dirichlet_f32(self.np_random, cfg.root_dirichlet_alpha, A, total_roots).reshape(total_roots, 1, A)
+            seed = self.np_random.choice(256)
+            u = self.np_random.random_sample(total_roots)[mine] if turn == "sample" else None
+            if self.speculate_noise:   # the next agent's noise draw overlaps this turn's enqueue (used only if np_random is untouched)
+                hostrng.speculate(self.np_random, cfg.root_dirichlet_alpha, A, total_roots)
+            plan.enqueue_turn(k, 1 if turn == "sample" else 0, int(seed), cfg, noise_epsilon, pad(noises[mine]), 1.0 / temperature,
+                              pad(u), greedy_epsilon, None if eps_u is None else pad(np.asarray(eps_u[k])),
+                              None if rand_act is None else pad(np.asarray(rand_act[k])), root_index_offset=start)
+        return plan, count
 
     # ---- reference simulation loop with the CUDA tree (any BaseNet) --------------------------------------------
     def _search_step_path(self, model, network_output, cur, factor, true_num_agents, device, sampled_tau, seed,

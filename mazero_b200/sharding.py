@@ -4,7 +4,9 @@ Trees are independent (private RNG seeded by the GLOBAL root index, cnode.cpp:57
 contiguous root slice `shard_range(B, r, world)` and passes `root_index_offset = start` to the search:
 results are identical to one `Tree_batch` over all B roots, whatever the number of ranks.  There is no
 collective inside the simulation loop; the only exchange is ONE all-gather of the packed readouts per
-search (root values, visit counts, sampled actions ...) so that the learner rank sees every root.
+search (root values, visit counts, sampled actions ...) so that the learner rank sees every root.  The per-agent loop of one
+environment step (`SampledMCTS.search_agents_sharded`) exchanges once per step: every agent's readouts and the turn results
+travel in one buffer (`merge_turn_shards`).
 """
 import numpy as np
 import torch
@@ -90,3 +92,39 @@ def merge_shards(blocks, spec_of, total_roots, world):
         d = split_packed(blocks[r], spec_of, shard_range(total_roots, 0, world)[1])
         parts.append({k: v[:count] for k, v in d.items()})
     return {k: np.concatenate([p[k] for p in parts], axis=0) for k in parts[0]}
+
+
+# ---- the sharded environment step (`SampledMCTS.search_agents_sharded`): ONE buffer per rank holds every agent's readouts and the
+# turn results, and ONE all-gather exchanges it -------------------------------------------------------------------------------------
+def split_turn_block(words, layout, roots):
+    """One rank's step buffer (1-D int32, `_DevicePlan.res_flat`) -> (per-agent readout dicts, dict of the turn fields).
+    layout = (readout_spec, agent_offsets, turn_fields) as `_DevicePlan.turn_layout()` gives it: the word offset of each agent's
+    packed readout block, and (name, dtype, shape, word offset) of every turn field.  8-byte fields are copied out of the int32 words
+    (never viewed at a 4-byte boundary), so their bits are kept whatever the buffer's alignment."""
+    readout_spec, agent_offsets, turn_fields = layout
+    n = sum(int(np.prod(shp)) for _, _, shp in readout_spec)
+    agents = [split_packed(words[o:o + n], readout_spec, roots) for o in agent_offsets]
+    turns = {}
+    for name, dt, shp, o in turn_fields:
+        dt = np.dtype(dt)
+        w = int(np.prod(shp)) * dt.itemsize // 4
+        assert dt.itemsize == 4 or o % 2 == 0, f"{name}: {dt} field at the odd word offset {o}"
+        assert o + w <= len(words), f"{name}: past the end of the block"
+        turns[name] = np.ascontiguousarray(words[o:o + w]).view(dt).reshape(shp)
+        assert turns[name].shape[0] == roots
+    return agents, turns
+
+
+def merge_turn_shards(blocks, layout, total_roots, world):
+    """blocks[r] = rank r's step buffer (padded to the largest shard); returns (per-agent readout dicts, turn-field dict) for ALL
+    roots in global root order, the padding rows dropped."""
+    rows = shard_range(total_roots, 0, world)[1]
+    assert len(blocks) == world and all(len(b) % 2 == 0 for b in blocks), "step buffers are whole 8-byte words"
+    parts = []
+    for r in range(world):
+        _, count = shard_range(total_roots, r, world)
+        agents, turns = split_turn_block(blocks[r], layout, rows)
+        parts.append(([{k: v[:count] for k, v in d.items()} for d in agents], {k: v[:count] for k, v in turns.items()}))
+    cat = lambda ds: {k: np.concatenate([d[k] for d in ds], axis=0) for k in ds[0]}
+    agents = [cat([p[0][t] for p in parts]) for t in range(len(parts[0][0]))]
+    return agents, cat([p[1] for p in parts])
