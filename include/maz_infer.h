@@ -23,7 +23,8 @@ int maz_dbg_umma_gemm(const float *a, const void *w_packed, float *out, int n, i
 /* Everything one launch of the fused recurrent_inference kernel needs.  All pointers are DEVICE pointers.
  * Fixed architecture (config/smac/__init__.py:15-27): hidden 128 per agent, 3 encoder layers x 8 heads,
  * dim_feedforward 128, fc_dynamic [128,128], GNN hidden 64, fc_policy [32], support 11; agents N <= 32,
- * actions A <= 48.  Weight packing: see mazero_b200/fused.py (pack_weights). */
+ * actions A <= 128 (KA > 48 launches the wide instances of the small-batch and the two-tiles-in-flight kernels; the first-generation
+ * kernel, tc_layout 0, takes A <= 48 and returns MAZ_ERR_UNSUPPORTED above).  Weight packing: see mazero_b200/fused.py (pack_weights). */
 #define MAZ_INFER_NCHUNK 32
 typedef struct maz_infer_desc {
     int B, N, A, KA, NAP;        /* roots, agents, actions, A rounded up to 16 (twice) */

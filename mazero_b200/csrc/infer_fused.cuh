@@ -64,7 +64,7 @@ struct Pipe {
 
 // one weight chunk: D[dst] (+)= A[a_addr (row length a_K)] * W_c^T  (n_out columns).  MMA thread only; not inlined
 // (called 32 times; small code = warm instruction cache).
-__device__ __noinline__ void mma_chunk(Pipe &p, uint32_t dst, uint32_t a_addr, uint32_t a_K, uint32_t n_out, uint32_t accum)
+static __device__ __noinline__ void mma_chunk(Pipe &p, uint32_t dst, uint32_t a_addr, uint32_t a_K, uint32_t n_out, uint32_t accum)
 {
     const int c = p.c, s = c % NSLOT;
     mbar_wait(&p.full[s], (c / NSLOT) & 1);
@@ -219,7 +219,7 @@ __device__ __forceinline__ void tmem_store_cols(uint32_t taddr, const float (&v)
 }
 
 // x0 = relu(acc + b_in) + pos[agent]  -> TMEM X (fp32) and operand tile (bf16)
-__device__ __noinline__ void epi_inproj(uint32_t trow, uint32_t sb, uint32_t spos, uint32_t tile)
+static __device__ __noinline__ void epi_inproj(uint32_t trow, uint32_t sb, uint32_t spos, uint32_t tile)
 {
     const Thr t;
     const int c = t.part * CP;
@@ -238,7 +238,7 @@ __device__ __noinline__ void epi_inproj(uint32_t trow, uint32_t sb, uint32_t spo
 }
 
 // f = relu(acc + b) -> operand tile
-__device__ __noinline__ void epi_bias_relu(uint32_t trow, uint32_t sb, uint32_t tile)
+static __device__ __noinline__ void epi_bias_relu(uint32_t trow, uint32_t sb, uint32_t tile)
 {
     const Thr t;
     const int c = t.part * CP;
@@ -252,7 +252,7 @@ __device__ __noinline__ void epi_bias_relu(uint32_t trow, uint32_t sb, uint32_t 
 
 // y = LN(acc + bias) * g + be over the 128 TMEM columns at `tcol`; optional ReLU (mlp()); optional fp32 copy
 // into the TMEM-resident residual stream X; always a bf16 copy into the operand tile.
-__device__ __noinline__ void epi_ln128(uint32_t trow, uint32_t tcol, uint32_t sb, uint32_t sg, uint32_t sbe, int relu_after,
+static __device__ __noinline__ void epi_ln128(uint32_t trow, uint32_t tcol, uint32_t sb, uint32_t sg, uint32_t sbe, int relu_after,
                                        int store_x, uint32_t tile, uint32_t aRed)
 {
     const Thr t;
@@ -327,7 +327,7 @@ __device__ __forceinline__ void attention_head_small(uint32_t trow, uint32_t sb,
     store_cols(tile, row, hh * HD, H, o);
 }
 
-__device__ __noinline__ void epi_attention(uint32_t trow, uint32_t sb, int N, int root_lane0, uint32_t tile, uint32_t scratch)
+static __device__ __noinline__ void epi_attention(uint32_t trow, uint32_t sb, int N, int root_lane0, uint32_t tile, uint32_t scratch)
 {
     const Thr t;
     const uint32_t kv = scratch + (uint32_t)(t.part * 4 + t.quad) * 2048u;   // this warp's 32 x (K16 | V16) bf16 rows
@@ -401,7 +401,7 @@ __device__ __noinline__ void epi_attention(uint32_t trow, uint32_t sb, int N, in
 }
 
 // next_hidden = acc + b + hidden (fp32 residual straight from the pool); fp32 to global, bf16 to the tile
-__device__ __noinline__ void epi_next_hidden(uint32_t trow, uint32_t sb, const float *__restrict__ hrow, float *__restrict__ nh,
+static __device__ __noinline__ void epi_next_hidden(uint32_t trow, uint32_t sb, const float *__restrict__ hrow, float *__restrict__ nh,
                                              int valid, uint32_t tile)
 {
     const Thr t;
@@ -426,7 +426,7 @@ __device__ __noinline__ void epi_next_hidden(uint32_t trow, uint32_t sb, const f
 // head == 1: mean-pool over the agents, 64 -> 11 head (V weights at sb + 128 floats, bias after), support
 //            transform; partial logits of the column parts are combined through `scratch` (shared, 24 KB);
 //            the scalar is returned by the part-0 thread of every row (0 elsewhere).
-__device__ __noinline__ float epi_gnn(uint32_t trow, uint32_t sb, int N, int root_lane0, int head, uint32_t tile, uint32_t aRed,
+static __device__ __noinline__ float epi_gnn(uint32_t trow, uint32_t sb, int N, int root_lane0, int head, uint32_t tile, uint32_t aRed,
                                       uint32_t scratch)
 {
     const Thr t;
@@ -514,7 +514,7 @@ __device__ __noinline__ float epi_gnn(uint32_t trow, uint32_t sb, int N, int roo
 }
 
 // policy hidden: p1 = relu(LN(acc + b) * g + be) over 32 columns -> operand tile (K = 32)
-__device__ __noinline__ void epi_policy_hidden(uint32_t trow, uint32_t sp, uint32_t tile, uint32_t aRed)
+static __device__ __noinline__ void epi_policy_hidden(uint32_t trow, uint32_t sp, uint32_t tile, uint32_t aRed)
 {
     const Thr t;
     const int c = t.part * PP;
@@ -539,7 +539,7 @@ __device__ __noinline__ void epi_policy_hidden(uint32_t trow, uint32_t sp, uint3
 // policy logits -> softmax -> probs, beta = probs^(1/tau) renormalised (mcts_sampled.py:158-161), greedy action.
 // Executed by the part-0 warps only (A <= 48 columns), as three rolled passes over 16-column TMEM chunks
 // (small code: this runs once per kernel, see issue_chunk's note on instruction fetch).
-__device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, uint32_t sb2, int valid, int root, int agent)
+static __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, uint32_t sb2, int valid, int root, int agent)
 {
     const int A = d.A, NAP = d.NAP;
     float m = -INFINITY;
@@ -596,7 +596,7 @@ __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, uint32
 }
 
 // fp32 pool row -> bf16 operand tile (K = 128), my 32 columns
-__device__ __noinline__ void gather_hidden(const float *__restrict__ hrow, int valid, uint32_t tile)
+static __device__ __noinline__ void gather_hidden(const float *__restrict__ hrow, int valid, uint32_t tile)
 {
     const Thr t;
     const int c = t.part * CP;
@@ -609,6 +609,7 @@ __device__ __noinline__ void gather_hidden(const float *__restrict__ hrow, int v
     store_cols(tile, t.row, c, H, v);
 }
 
+#ifndef MAZ_FUSED_NO_KERNEL   // (translation units that only need the device functions define it)
 __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference(const __grid_constant__ Desc d)
 {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -847,6 +848,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference(const __gri
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
+#endif  // MAZ_FUSED_NO_KERNEL
 
 }  // namespace fused
 }  // namespace maz

@@ -78,6 +78,12 @@ constexpr int Y_R = 0, Y_V = TM * GH;                            // layer-2 feat
 constexpr int PL0 = 2 * TM * LDG;                                // policy logits                          [TM][48]
 static_assert((PL0 + TM * 48) * 4 <= TM * LDQ, "heads scratch must fit in the q|k|v region");
 static_assert(2 * TM * GH * 4 <= 2 * TM * LDA, "layer-2 features must fit in the X + T tiles");
+// The WIDE variant (template argument W = true, 48 < KA <= 128) keeps this map.  The one-hot tile region holds one int per row
+// (the row's action, -1 = none) and the one-hot MMA operand is built in registers (gemm_onehot); the policy logits, [TM][128]
+// fp32, go to the X + T tiles once the layer-2 features there have been consumed (stage_heads2).
+constexpr int KA_NARROW = 48, KA_WIDE = 128;
+static_assert(TM * 4 <= TM * LDO, "wide variant: the row actions must fit in the one-hot tile region");
+static_assert(TM * KA_WIDE * 4 <= 2 * TM * LDA, "wide variant: the policy logits must fit in the X + T tiles");
 
 using Desc = ::maz_infer_desc;
 
@@ -191,7 +197,7 @@ __device__ __forceinline__ void gemm_fixed(float (&acc)[NT][4], const Thr &th, u
         }
     }
 }
-// the same with a run-time K (the one-hot operand: K = KA in {16, 32, 48})
+// the same with a run-time K (the one-hot operand of the narrow variant: K = KA in {16, 32, 48})
 template <int NT>
 __device__ __forceinline__ void gemm_rt(float (&acc)[NT][4], const Thr &th, uint32_t a_tile, int lda, uint32_t w_slot, int ldw, int n0, int K)
 {
@@ -207,6 +213,40 @@ __device__ __forceinline__ void gemm_rt(float (&acc)[NT][4], const Thr &th, uint
             mma16816(acc[2 * p], a, b[p][0], b[p][1]);
             mma16816(acc[2 * p + 1], a, b[p][2], b[p][3]);
         }
+    }
+}
+// the same product for the wide variant: the A operand is the one-hot matrix of the row actions actA (row th.rA) and actB (row
+// th.rB), built in registers -- fragment word i holds rows rA (i even) / rB (i odd), columns k0 + 2t (+8 for i >= 2) and +1
+template <int NT>
+__device__ __forceinline__ void gemm_onehot(float (&acc)[NT][4], const Thr &th, int actA, int actB, uint32_t w_slot, int ldw, int n0, int K)
+{
+    const uint32_t wa = th.w_addr(w_slot, ldw, n0);
+#pragma unroll 1
+    for (int k0 = 0; k0 < K; k0 += 16) {
+        const int c = k0 + 2 * th.t;
+        uint32_t a[4], b[NT / 2][4];
+        a[0] = pack2(c == actA ? 1.f : 0.f, c + 1 == actA ? 1.f : 0.f);
+        a[1] = pack2(c == actB ? 1.f : 0.f, c + 1 == actB ? 1.f : 0.f);
+        a[2] = pack2(c + 8 == actA ? 1.f : 0.f, c + 9 == actA ? 1.f : 0.f);
+        a[3] = pack2(c + 8 == actB ? 1.f : 0.f, c + 9 == actB ? 1.f : 0.f);
+#pragma unroll
+        for (int p = 0; p < NT / 2; ++p) ldsm4(wa + (uint32_t)(16 * p) * ldw + 2u * k0, b[p]);
+#pragma unroll
+        for (int p = 0; p < NT / 2; ++p) {
+            mma16816(acc[2 * p], a, b[p][0], b[p][1]);
+            mma16816(acc[2 * p + 1], a, b[p][2], b[p][3]);
+        }
+    }
+}
+// acc += [h | onehot(a)] one-hot part: the one-hot tile (narrow) or the row actions (wide)
+template <bool W, int NT>
+__device__ __forceinline__ void gemm_action(float (&acc)[NT][4], const Thr &th, uint32_t sb, uint32_t w_slot, int ldw, int n0, int K)
+{
+    if constexpr (W) {
+        const int actA = __float_as_int(lds1v(sb + OFF_ONE + 4u * th.rA)), actB = __float_as_int(lds1v(sb + OFF_ONE + 4u * th.rB));
+        gemm_onehot<NT>(acc, th, actA, actB, w_slot, ldw, n0, K);
+    } else {
+        gemm_rt<NT>(acc, th, sb + OFF_ONE, LDO, w_slot, ldw, n0, K);
     }
 }
 
@@ -352,7 +392,9 @@ __device__ __forceinline__ RowInfo row_info(int r)
 }
 
 // ---- stages (not inlined: the kernel is one long straight line, small code keeps the instruction cache warm) ----------
-// fp32 pool rows -> bf16 tile HH; one-hot joint action -> tile One.  Thread (row = tid/8, 16 columns each).
+// fp32 pool rows -> bf16 tile HH; one-hot joint action -> tile One (wide variant: the row's action).  Thread (row = tid/8, 16
+// columns each).
+template <bool W>
 static __device__ __noinline__ void stage_gather(const Desc &d, const SimIo io)
 {
     HSM_DECL;
@@ -382,7 +424,9 @@ static __device__ __noinline__ void stage_gather(const Desc &d, const SimIo io)
     uint4 *dst = reinterpret_cast<uint4 *>(hsm + OFF_HH + (size_t)r * LDA + part * 32);
     dst[0] = make_uint4(w[0], w[1], w[2], w[3]);
     dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
-    if (part * 8 < d.KA) {               // 8 one-hot columns per thread
+    if constexpr (W) {
+        if (part == 0) *reinterpret_cast<int *>(hsm + OFF_ONE + (size_t)r * 4) = action;
+    } else if (part * 8 < d.KA) {        // 8 one-hot columns per thread
         const int c0 = part * 8;
         uint32_t o[4];
 #pragma unroll
@@ -392,6 +436,7 @@ static __device__ __noinline__ void stage_gather(const Desc &d, const SimIo io)
 }
 
 // x0 = relu(W_in [h | onehot] + b) + pos[agent]  -> residual fragment x, bf16 tile X
+template <bool W>
 static __device__ __noinline__ void stage_inproj(const Desc &d, Ring &ring, float (&xio)[NT][4])
 {
     const Thr th;
@@ -403,7 +448,7 @@ static __device__ __noinline__ void stage_inproj(const Desc &d, Ring &ring, floa
     gemm_fixed<NT, 8>(x, th, sb + OFF_HH, LDA, w, LDA, n0);
     ring.release(th.lane);
     w = ring.acquire();
-    gemm_rt<NT>(x, th, sb + OFF_ONE, LDO, w, ldo, n0, d.KA);
+    gemm_action<W, NT>(x, th, sb, w, ldo, n0, d.KA);
     ring.release(th.lane);
     add_bias<NT>(x, th, sb + OFF_P + 4u * d.o_bin, n0);
     const uint32_t pA = sb + OFF_P + 4u * (d.o_pos + row_info(th.rA).agent * H), pB = sb + OFF_P + 4u * (d.o_pos + row_info(th.rB).agent * H);
@@ -618,6 +663,7 @@ static __device__ __noinline__ void stage_linear_relu(Ring &ring, uint32_t bias)
 
 // fc_dynamic (model.py:262-268): [h | onehot | attn] -> Linear LN ReLU -> Linear LN ReLU -> Linear, + h; next_hidden to
 // global (fp32) and to tile T (bf16)
+template <bool W>
 static __device__ __noinline__ void stage_dynamics(const Desc &d, Ring &ring, const SimIo io)
 {
     const Thr th;
@@ -630,7 +676,7 @@ static __device__ __noinline__ void stage_dynamics(const Desc &d, Ring &ring, co
     gemm_fixed<NT, 8>(acc, th, sb + OFF_HH, LDA, w, LDA, n0);        // h
     ring.release(th.lane);
     w = ring.acquire();
-    gemm_rt<NT>(acc, th, sb + OFF_ONE, LDO, w, ldo, n0, d.KA);       // one-hot action
+    gemm_action<W, NT>(acc, th, sb, w, ldo, n0, d.KA);               // one-hot action
     ring.release(th.lane);
     w = ring.acquire();
     gemm_fixed<NT, 8>(acc, th, sb + OFF_X, LDA, w, LDA, n0);         // attention output
@@ -749,6 +795,7 @@ __device__ __forceinline__ void gnn_phase_c(const Thr &th, uint32_t stat, float 
 
 // heads, first layers, ONE stage: reward GNN layer 1 on [next_hidden | onehot], value GNN layer 1 and fc_policy.0 on
 // next_hidden.  Outputs: X[:, 0:64] = reward features, X[:, 64:128] = value features, Ph = relu(LN(policy hidden)).
+template <bool W>
 static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
 {
     const Thr th;
@@ -760,7 +807,7 @@ static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
     gemm_fixed<NT, 8>(aR, th, sb + OFF_T, LDA, w, LDA, n0);
     ring.release(th.lane);
     w = ring.acquire();
-    gemm_rt<NT>(aR, th, sb + OFF_ONE, LDO, w, ldo, n0, d.KA);
+    gemm_action<W, NT>(aR, th, sb, w, ldo, n0, d.KA);
     ring.release(th.lane);
     w = ring.acquire();
     gemm_fixed<NT, 8>(aV, th, sb + OFF_T, LDA, w, LDA, n0);
@@ -827,70 +874,19 @@ __device__ __forceinline__ float support_to_scalar(const float (&v)[SUP])
     return out;
 }
 
-// heads, second layers + outputs, ONE stage: reward / value GNN layer 2 -> mean over agents -> 64->11 head -> scalar;
-// fc_policy.3 -> softmax / beta / greedy (mcts_sampled.py:158-161).
-static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, const SimIo io, long long *hs_clk)
+// policy outputs from the fp32 logits at shared address PL ([TM][LD]): 8 threads per row (softmax, beta, greedy).  Every thread
+// keeps its (at most LD / 8) logits in registers: one batch of loads, two 8-lane reductions, one batch of stores.
+template <int LD>
+__device__ __forceinline__ void policy_outputs(const Desc &d, const SimIo io, uint32_t PL, long long *hs_clk, int &hs_n)
 {
-    const Thr th;
-    const uint32_t sb = sbase();
-    const int n0 = CW * th.nq, ldg = (GH + PAD) * 2;
     const int N = d.N, A = d.A, tid = threadIdx.x;
-    int hs_n = 40;
 #define HS() \
     if (hs_clk && hs_n < 64) hs_clk[hs_n++] = clock64();
-    HS();
-    float aR[NT][4], aV[NT][4], aP[2][4];
-    zero<NT>(aR); zero<NT>(aV); zero<2>(aP);
-    uint32_t w = ring.acquire();
-    gemm_fixed<NT, 4>(aR, th, sb + OFF_X, LDA, w, ldg, n0);
-    ring.release(th.lane);
-    w = ring.acquire();
-    gemm_fixed<NT, 4>(aV, th, sb + OFF_X + GH * 2, LDA, w, ldg, n0);
-    ring.release(th.lane);
-    w = ring.acquire();
-    const int pc0 = 16 * th.nq;                                    // policy logit columns [16*nq, +16) when < NAP
-    if (pc0 < d.NAP) gemm_fixed<2, 2>(aP, th, sb + OFF_PH, LDP, w, LDP, pc0);
-    ring.release(th.lane);
-    const uint32_t G = sb + OFF_Q, stat = sb + OFF_STAT, pr = sb + OFF_P + 4u * (d.o_rg + 128), pvv = sb + OFF_P + 4u * (d.o_vg + 128);
-    const uint32_t PL = G + 4u * PL0;
-    HS();
-    // phase A
-    gnn_phase_a(aR, th, G + 4u * G_R, pr);
-    gnn_phase_a(aV, th, G + 4u * G_V, pvv);
-    if (pc0 < d.NAP) {                                             // policy logits + bias -> fp32 scratch [TM][48]
-        const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
-#pragma unroll
-        for (int tl = 0; tl < 2; ++tl) {
-            const int c = pc0 + 8 * tl + 2 * th.t;
-            const float2 bb = ldp2(b2 + 4u * c);
-            sts2f(PL + 4u * (th.rA * 48 + c), aP[tl][0] + bb.x, aP[tl][1] + bb.y);
-            sts2f(PL + 4u * (th.rB * 48 + c), aP[tl][2] + bb.x, aP[tl][3] + bb.y);
-        }
-    }
-    cta_sync();
-    HS();
-    // phase B
-    const int r0A = row_info(th.rA).r0, r0B = row_info(th.rB).r0;
-    float yR[GT][4], yV[GT][4];
-    gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, N, r0A, r0B, yR);
-    gnn_phase_b(aV, th, G + 4u * G_V, pvv, stat + STAT_SET, N, r0A, r0B, yV);
-    // the raw (post-ReLU) layer-2 features, fp32 -> Y in the X + T tiles (free since the GEMMs above)
-    const uint32_t YB = sb + OFF_X;
-#pragma unroll
-    for (int tl = 0; tl < GT; ++tl) {
-        const int f = FW * th.nq + 8 * tl + 2 * th.t;
-        sts2f(YB + 4u * (Y_R + th.rA * GH + f), yR[tl][0], yR[tl][1]);
-        sts2f(YB + 4u * (Y_R + th.rB * GH + f), yR[tl][2], yR[tl][3]);
-        sts2f(YB + 4u * (Y_V + th.rA * GH + f), yV[tl][0], yV[tl][1]);
-        sts2f(YB + 4u * (Y_V + th.rB * GH + f), yV[tl][2], yV[tl][3]);
-    }
-    HS();
-    if (tid < TM * 8) {   // policy outputs: 8 threads per row (softmax, beta, greedy); warp-uniform condition
-        // every thread keeps its (at most 6) logits in registers: one batch of loads, two 8-lane reductions, one batch of stores
-        constexpr int PA = 6;                                          // actions per thread: A <= 48
+    if (tid < TM * 8) {   // warp-uniform condition
+        constexpr int PA = LD / 8;                                     // actions per thread
         const int r = tid >> 3, sub = tid & 7;
         const RowInfo ri = row_info(r);
-        const uint32_t lg = PL + 4u * (r * 48);
+        const uint32_t lg = PL + 4u * (r * LD);
         float v[PA];
 #pragma unroll
         for (int i = 0; i < PA; ++i) v[i] = (sub + 8 * i < A) ? lds1v(lg + 4u * (sub + 8 * i)) : -INFINITY;
@@ -939,6 +935,76 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
             }
         }
     }
+#undef HS
+}
+
+// heads, second layers + outputs, ONE stage: reward / value GNN layer 2 -> mean over agents -> 64->11 head -> scalar;
+// fc_policy.3 -> softmax / beta / greedy (mcts_sampled.py:158-161).  The narrow variant stages the policy logits in the q|k|v
+// region and computes the policy outputs in phase B; the wide variant keeps its PB logit blocks per warp in registers until
+// phase D has consumed the layer-2 features and then uses the X + T tiles (one more barrier).
+template <bool W>
+static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, const SimIo io, long long *hs_clk)
+{
+    const Thr th;
+    const uint32_t sb = sbase();
+    const int n0 = CW * th.nq, ldg = (GH + PAD) * 2;
+    const int N = d.N, tid = threadIdx.x;
+    int hs_n = 40;
+#define HS() \
+    if (hs_clk && hs_n < 64) hs_clk[hs_n++] = clock64();
+    HS();
+    constexpr int PB = W ? (KA_WIDE / 16 + NQ - 1) / NQ : 1;          // 16-column logit blocks per warp
+    float aR[NT][4], aV[NT][4], aP[PB][2][4];
+    zero<NT>(aR); zero<NT>(aV);
+#pragma unroll
+    for (int bk = 0; bk < PB; ++bk) zero<2>(aP[bk]);
+    uint32_t w = ring.acquire();
+    gemm_fixed<NT, 4>(aR, th, sb + OFF_X, LDA, w, ldg, n0);
+    ring.release(th.lane);
+    w = ring.acquire();
+    gemm_fixed<NT, 4>(aV, th, sb + OFF_X + GH * 2, LDA, w, ldg, n0);
+    ring.release(th.lane);
+    w = ring.acquire();
+    const int pc0 = 16 * th.nq;                                    // policy logit columns [16*nq, +16) (+ 16*NQ*bk) when < NAP
+#pragma unroll
+    for (int bk = 0; bk < PB; ++bk)
+        if (pc0 + NQ * 16 * bk < d.NAP) gemm_fixed<2, 2>(aP[bk], th, sb + OFF_PH, LDP, w, LDP, pc0 + NQ * 16 * bk);
+    ring.release(th.lane);
+    const uint32_t G = sb + OFF_Q, stat = sb + OFF_STAT, pr = sb + OFF_P + 4u * (d.o_rg + 128), pvv = sb + OFF_P + 4u * (d.o_vg + 128);
+    const uint32_t PL = G + 4u * PL0;
+    HS();
+    // phase A
+    gnn_phase_a(aR, th, G + 4u * G_R, pr);
+    gnn_phase_a(aV, th, G + 4u * G_V, pvv);
+    if (!W && pc0 < d.NAP) {                                       // policy logits + bias -> fp32 scratch [TM][48]
+        const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
+#pragma unroll
+        for (int tl = 0; tl < 2; ++tl) {
+            const int c = pc0 + 8 * tl + 2 * th.t;
+            const float2 bb = ldp2(b2 + 4u * c);
+            sts2f(PL + 4u * (th.rA * 48 + c), aP[0][tl][0] + bb.x, aP[0][tl][1] + bb.y);
+            sts2f(PL + 4u * (th.rB * 48 + c), aP[0][tl][2] + bb.x, aP[0][tl][3] + bb.y);
+        }
+    }
+    cta_sync();
+    HS();
+    // phase B
+    const int r0A = row_info(th.rA).r0, r0B = row_info(th.rB).r0;
+    float yR[GT][4], yV[GT][4];
+    gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, N, r0A, r0B, yR);
+    gnn_phase_b(aV, th, G + 4u * G_V, pvv, stat + STAT_SET, N, r0A, r0B, yV);
+    // the raw (post-ReLU) layer-2 features, fp32 -> Y in the X + T tiles (free since the GEMMs above)
+    const uint32_t YB = sb + OFF_X;
+#pragma unroll
+    for (int tl = 0; tl < GT; ++tl) {
+        const int f = FW * th.nq + 8 * tl + 2 * th.t;
+        sts2f(YB + 4u * (Y_R + th.rA * GH + f), yR[tl][0], yR[tl][1]);
+        sts2f(YB + 4u * (Y_R + th.rB * GH + f), yR[tl][2], yR[tl][3]);
+        sts2f(YB + 4u * (Y_V + th.rA * GH + f), yV[tl][0], yV[tl][1]);
+        sts2f(YB + 4u * (Y_V + th.rB * GH + f), yV[tl][2], yV[tl][3]);
+    }
+    HS();
+    if constexpr (!W) policy_outputs<KA_NARROW>(d, io, PL, hs_clk, hs_n);
     HS();
     cta_sync();
     HS();
@@ -974,6 +1040,22 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     }
     cta_sync();
     HS();
+    if constexpr (W) {                                             // the layer-2 features are consumed: logits + bias -> X + T tiles
+        const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
+#pragma unroll
+        for (int bk = 0; bk < PB; ++bk) {
+            const int pc = pc0 + NQ * 16 * bk;
+            if (pc < d.NAP) {
+#pragma unroll
+                for (int tl = 0; tl < 2; ++tl) {
+                    const int c = pc + 8 * tl + 2 * th.t;
+                    const float2 bb = ldp2(b2 + 4u * c);
+                    sts2f(sb + OFF_X + 4u * (th.rA * KA_WIDE + c), aP[bk][tl][0] + bb.x, aP[bk][tl][1] + bb.y);
+                    sts2f(sb + OFF_X + 4u * (th.rB * KA_WIDE + c), aP[bk][tl][2] + bb.x, aP[bk][tl][3] + bb.y);
+                }
+            }
+        }
+    }
     // phase E: a half-warp per (root, head): lane k < 11 computes logit k of the 64 -> 11 head (weights from the padded copy:
     // conflict-free float4 rows), the 11 logits meet in the half-warp's first lane by shuffles, which applies
     // softmax . support -> inv_h and stores the scalar.  No barrier, no shared-memory round trip.
@@ -1008,6 +1090,10 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
         }
     }
     HS();
+    if constexpr (W) {
+        cta_sync();
+        policy_outputs<KA_WIDE>(d, io, sb + OFF_X, hs_clk, hs_n);
+    }
 #undef HS
 }
 
@@ -1055,7 +1141,8 @@ __device__ __forceinline__ void setup_head_copies(const Desc &d)
 }
 
 // one recurrent_inference of the CTA's tile: every stage after the gather (compute warps; row table, parameters and head
-// copies are set up).  `clk` (or NULL): SM-cycle timestamps of the stages, written by thread 0.
+// copies are set up).  `clk` (or NULL): SM-cycle timestamps of the stages, written by thread 0.  W: the wide variant (KA > 48).
+template <bool W>
 __device__ __forceinline__ void infer_stages(const Desc &d, const SimIo io, Ring &ring, long long *clk)
 {
     int ts_n = 2;
@@ -1063,7 +1150,7 @@ __device__ __forceinline__ void infer_stages(const Desc &d, const SimIo io, Ring
     if (clk && ts_n < 64) clk[ts_n++] = clock64();
     TS();
     float x[NT][4];
-    stage_inproj(d, ring, x);
+    stage_inproj<W>(d, ring, x);
     TS();
     const uint32_t pbase = sbase() + OFF_P;
 #pragma unroll 1
@@ -1081,16 +1168,17 @@ __device__ __forceinline__ void infer_stages(const Desc &d, const SimIo io, Ring
         TS();
     }
     TS();
-    stage_dynamics(d, ring, io);
+    stage_dynamics<W>(d, ring, io);
     TS();
-    stage_heads1(d, ring);
+    stage_heads1<W>(d, ring);
     TS();
-    stage_heads2(d, ring, io, clk);
+    stage_heads2<W>(d, ring, io, clk);
     TS();
 #undef TS
 }
 
 #ifndef MAZ_HMMA_NO_KERNEL
+template <bool W>
 __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference_small(const __grid_constant__ Desc d)
 {
     HSM_DECL;
@@ -1119,12 +1207,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference_small(const
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     const SimIo io = io_from_desc(d);
-    stage_gather(d, io);
+    stage_gather<W>(d, io);
     if (clk) clk[1] = clock64();
     mbar_wait(&bar_vec, 0);          // parameters resident
     setup_head_copies(d);
     cta_sync();
-    infer_stages(d, io, ring, clk);
+    infer_stages<W>(d, io, ring, clk);
 }
 #endif  // MAZ_HMMA_NO_KERNEL
 

@@ -236,7 +236,7 @@ __device__ __forceinline__ void row_stats_pr(const Thr &t, uint32_t aRed, float 
 // `trow`: TMEM address of the tile's ACC0 at this warp's lanes; `oh`: this row's column of the one-hot weight block (or NULL).
 
 // x0 = relu(acc + b_in + W_a[:, action]) + pos[agent] -> sX
-__device__ __noinline__ void epi_inproj(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ oh, const float *__restrict__ pos,
+static __device__ __noinline__ void epi_inproj(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ oh, const float *__restrict__ pos,
                                         uint32_t aX)
 {
     const Thr t;
@@ -251,7 +251,7 @@ __device__ __noinline__ void epi_inproj(uint32_t trow, const float *__restrict__
     store_cols(aX, t.row, c, H, v);
 }
 // acc + b -> bf16 tile (V of the attention; relu != 0: relu(linear1))
-__device__ __noinline__ void epi_bias(uint32_t trow, const float *__restrict__ pb, int relu, uint32_t tile)
+static __device__ __noinline__ void epi_bias(uint32_t trow, const float *__restrict__ pb, int relu, uint32_t tile)
 {
     const Thr t;
     const int c = t.part * 32;
@@ -266,7 +266,7 @@ __device__ __noinline__ void epi_bias(uint32_t trow, const float *__restrict__ p
     store_cols(tile, t.row, c, H, v);
 }
 // y = LN(acc + b [+ oh] [+ x from res_tile]) * g + be, optional ReLU -> dst tile (bf16)
-__device__ __noinline__ void epi_ln(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ pg, const float *__restrict__ pbe,
+static __device__ __noinline__ void epi_ln(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ pg, const float *__restrict__ pbe,
                                     const float *__restrict__ oh, uint32_t res_tile, int relu_after, uint32_t dst_tile, uint32_t aRed, int dbg = 0)
 {
     const Thr t;
@@ -302,7 +302,7 @@ __device__ __noinline__ void epi_ln(uint32_t trow, const float *__restrict__ pb,
 //   layout), S[32 x 32] = Q K^T on 8 MMAs, keys of other roots masked, row softmax on the fragments (a row's 32 scores sit in
 //   the 4 lanes of a quad), P as bf16 A fragments, O[32 x 16] = P V on 8 MMAs with V fragments by ldmatrix.trans from aT.
 // Rows beyond the last whole root of the warp form a pseudo-root of their own (finite garbage, never stored anywhere).
-__device__ __noinline__ void epi_attention(uint32_t trow, uint32_t aT, const float *__restrict__ pqk, int N, uint32_t scratch, int half)
+static __device__ __noinline__ void epi_attention(uint32_t trow, uint32_t aT, const float *__restrict__ pqk, int N, uint32_t scratch, int half)
 {
     const Thr t;
     const int l = t.lane, m = l >> 3;
@@ -428,7 +428,7 @@ __device__ __noinline__ void epi_attention(uint32_t trow, uint32_t aT, const flo
 }
 
 // next_hidden = acc + b + hidden (fp32 residual straight from the pool); fp32 to global, bf16 to the tile
-__device__ __noinline__ void epi_next_hidden(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ hrow, float *__restrict__ nh,
+static __device__ __noinline__ void epi_next_hidden(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ hrow, float *__restrict__ nh,
                                              int valid, uint32_t tile)
 {
     const Thr t;
@@ -449,7 +449,7 @@ __device__ __noinline__ void epi_next_hidden(uint32_t trow, const float *__restr
     store_cols(tile, t.row, c, H, v);
 }
 // fp32 pool row -> bf16 operand tile (K = 128), my 32 columns
-__device__ __noinline__ void gather_hidden(const float *__restrict__ hrow, int valid, uint32_t tile)
+static __device__ __noinline__ void gather_hidden(const float *__restrict__ hrow, int valid, uint32_t tile)
 {
     const Thr t;
     const int c = t.part * 32;
@@ -499,7 +499,7 @@ __device__ __forceinline__ void root_sum(float (&v)[NV], int lane, int lo, int N
 //            16 features of ITS row to 11 partial logits; the four column parts of a row are combined through shared memory,
 //            the rows of a root by the part-0 warp (root_sum over 11 values instead of 16 features x 4 parts).  The scalar is
 //            returned by the part-0 thread of every row.
-__device__ __noinline__ float epi_gnn(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ oh, int N, int root_lane0, int head,
+static __device__ __noinline__ float epi_gnn(uint32_t trow, const float *__restrict__ pb, const float *__restrict__ oh, int N, int root_lane0, int head,
                                       uint32_t tile, uint32_t aRed, uint32_t scratch, long long *clk = nullptr)
 {
     const Thr t;
@@ -590,7 +590,7 @@ __device__ __noinline__ float epi_gnn(uint32_t trow, const float *__restrict__ p
 }
 
 // policy hidden: p1 = relu(LN(acc + b) * g + be) over 32 columns -> operand tile (K = 32)
-__device__ __noinline__ void epi_policy_hidden(uint32_t trow, const float *__restrict__ pp, uint32_t tile, uint32_t aRed)
+static __device__ __noinline__ void epi_policy_hidden(uint32_t trow, const float *__restrict__ pp, uint32_t tile, uint32_t aRed)
 {
     const Thr t;
     const int c = t.part * PP;
@@ -610,34 +610,45 @@ __device__ __noinline__ void epi_policy_hidden(uint32_t trow, const float *__res
 }
 
 // policy logits -> softmax -> probs, beta = probs^(1/tau) renormalised (mcts_sampled.py:158-161), greedy action.
-// Column part p owns logits [16p, 16p + 16) of its row (parts beyond the padded action count idle).  Every part reduces its own
-// columns (local maximum m_p, argmax, sum of exp(v - m_p), sum of exp((v - m_p)/tau)); ONE exchange through shared memory (ex: 8 KB)
-// combines them: M = max m_p, s = sum s_p exp(m_p - M).
-__device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const float *__restrict__ pb2, int valid, int root, int agent,
+// Column part p owns logits [NV p, NV p + NV) of its row, NV = 16 (narrow, NAP <= 64) or 32 (W: the wide variant, NAP <= 128; two
+// 16-column TMEM blocks per part); parts beyond the padded action count idle.  Every part reduces its own columns (local maximum
+// m_p, argmax, sum of exp(v - m_p), sum of exp((v - m_p)/tau)); ONE exchange through shared memory (ex: 8 KB) combines them:
+// M = max m_p, s = sum s_p exp(m_p - M).  The parts are in column order, so the first part with the maximum holds the first
+// maximum.  `stage`: the joint-mode staging area, 32 x 48 floats per quadrant from `stage` (narrow), 32 x 128 floats per quadrant in
+// the two (free) sT operand tiles from `stage` = tile 0's sT (wide).
+template <bool W>
+static __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const float *__restrict__ pb2, int valid, int root, int agent,
                                             uint32_t ex, uint32_t stage, long long *clk = nullptr)
 {
     const Thr t;
 #define SUBTS(i) if (clk) clk[i] = clock64();
     SUBTS(0)
-    const int A = d.A, cc = t.part * 16;
+    constexpr int NV = W ? 32 : 16;
+    const int A = d.A, cc = t.part * NV;
     const bool active = cc < d.NAP;                  // warp-uniform (tcgen05.ld is warp-collective)
     const bool unit_tau = (d.inv_tau == 1.0f);
-    float v[16];
+    float v[NV];
     float m = -INFINITY, s = 0.f, sbeta = 0.f;
     int am = 0;
     if (active) {
-        tmem_ld16(trow + TM_A0 + cc, v);
-        add_gvec(v, pb2 + cc);
 #pragma unroll
-        for (int i = 0; i < 16; ++i)
+        for (int b = 0; b < NV / 16; ++b) {
+            float (&vb)[16] = *reinterpret_cast<float (*)[16]>(v + 16 * b);
+            if (b == 0 || cc + 16 * b < d.NAP) {    // (warp-uniform)
+                tmem_ld16(trow + TM_A0 + cc + 16 * b, vb);
+                add_gvec(vb, pb2 + cc + 16 * b);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < NV; ++i)
             if (cc + i < A && v[i] > m) { m = v[i]; am = cc + i; }
         if (valid && d.logits_out) {
 #pragma unroll
-            for (int i = 0; i < 16; ++i)
+            for (int i = 0; i < NV; ++i)
                 if (cc + i < A) d.logits_out[((size_t)root * d.N + agent) * A + cc + i] = v[i];
         }
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
+        for (int i = 0; i < NV; ++i) {
             const float e = (cc + i < A) ? __expf(v[i] - m) : 0.f;
             v[i] = e;
             s += e;
@@ -671,7 +682,8 @@ __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const 
         // joint mode: the rows of a quadrant are consecutive (root, agent) pairs, i.e. ONE contiguous block of probs / beta in
         // global memory: stage the quadrant's block in shared memory and copy it out with coalesced stores (a row-per-thread
         // store touches 32 sectors per instruction: ~13 k cycles per tile at 27m).  tau = 1: beta == probs, one pass.
-        const uint32_t st = stage + (uint32_t)t.quad * (32u * 48u * 4u);
+        const uint32_t st = W ? stage + (uint32_t)(t.quad >> 1) * 2u * TILE_BYTES + (uint32_t)(t.quad & 1) * (32u * 128u * 4u)
+                              : stage + (uint32_t)t.quad * (32u * 48u * 4u);
         const int rpw = 32 / d.N;
         const int q_root0 = __shfl_sync(0xffffffffu, root, 0);          // lane 0 holds the quadrant's first root
         const int nroots = max(0, min(rpw, d.B - q_root0));
@@ -684,7 +696,7 @@ __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const 
             if (pass) named_bar_sync(1 + t.quad, 128);                   // pass 0 has been copied out
             if (active) {
 #pragma unroll
-                for (int i = 0; i < 16; ++i)
+                for (int i = 0; i < NV; ++i)
                     if (cc + i < A) sts1f(st + (uint32_t)(t.lane * A + cc + i) * 4u, pass == 0 ? v[i] * invs : __powf(v[i], d.inv_tau) * invb);
             }
             SUBTS(4)
@@ -705,7 +717,7 @@ __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const 
     if (active && valid && ta >= 0) {
         float *po = d.probs + ((size_t)root * d.Nt + ta) * A, *bo = d.beta + ((size_t)root * d.Nt + ta) * A;
 #pragma unroll
-        for (int i = 0; i < 16; ++i)
+        for (int i = 0; i < NV; ++i)
             if (cc + i < A) {
                 po[cc + i] = v[i] * invs;
                 bo[cc + i] = (unit_tau ? v[i] * invs : __powf(v[i], d.inv_tau) * invb);
@@ -713,6 +725,8 @@ __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow, const 
     }
 }
 
+// W: the wide variant (48 < NAP <= 128), which differs in the policy output epilogue only (epi_policy_out)
+template <bool W>
 __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference_twin(const __grid_constant__ Desc d)
 {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -922,7 +936,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_recurrent_inference_twin(const 
         for (int tt = 0; tt < 2; ++tt) {
             TILE_VARS
             WAIT_MMA();
-            epi_policy_out(d, trow, pv + 96, valid, root, agent, aRed, aScr, ts_on ? d.dbg_clock + 160 + 16 * tt : nullptr);
+            epi_policy_out<W>(d, trow, pv + 96, valid, root, agent, aRed, W ? aTile + TILE_BYTES : aScr,
+                              ts_on ? d.dbg_clock + 160 + 16 * tt : nullptr);
             TS();
         }
 #undef STAGE

@@ -15,6 +15,10 @@ using namespace maz::umma;
 
 extern "C" const char *maz_last_error(void);
 namespace maz { int set_last_error(int code, const std::string &msg); bool pdl_enabled(); int pdl_mask(); }
+namespace maz { namespace twin {     // maz_infer_wide.cu: the wide instance of the two-tiles-in-flight kernel
+const void *wide_kernel();
+cudaError_t launch_wide(const cudaLaunchConfig_t &cfg, const maz_infer_desc &d);
+} }
 
 // ---------------------------------------------------------------------------------------------------------
 // Self-test kernel: one GEMM stage exactly as the fused kernel runs it.
@@ -97,12 +101,15 @@ extern "C" int maz_infer_configure(int vec_floats, int ka);
 extern "C" int maz_infer_recurrent(const maz_infer_desc *d, void *stream)
 {
     if (!d) return set_last_error(1, "maz_infer_recurrent: NULL descriptor");
-    if (d->B <= 0 || d->N <= 0 || d->N > 32 || d->A <= 0 || d->A > 48 || d->KA % 16 || d->KA < d->A || d->NAP != d->KA)
-        return set_last_error(3, "maz_infer_recurrent: unsupported shape (agents <= 32, actions <= 48)");
+    if (d->B <= 0 || d->N <= 0 || d->N > 32 || d->A <= 0 || d->A > hmma::KA_WIDE || d->KA % 16 || d->KA < d->A || d->KA > hmma::KA_WIDE ||
+        d->NAP != d->KA)
+        return set_last_error(3, "maz_infer_recurrent: unsupported shape (agents <= 32, actions <= 128)");
+    if (d->tc_layout == 0 && d->A > hmma::KA_NARROW)
+        return set_last_error(3, "maz_infer_recurrent: the first-generation kernel (tc_layout 0) supports at most 48 actions; use tc_layout 1");
     if (!d->pool || !d->actions || !d->next_hidden || !d->reward || !d->value || !d->probs || !d->beta || !d->wpk || !d->vec)
         return set_last_error(1, "maz_infer_recurrent: NULL tensor");
     if (d->vec_floats <= 0 || d->vec_floats % 4) return set_last_error(1, "maz_infer_recurrent: vec_floats must be a positive multiple of 4");
-    const bool tw = d->tc_layout == 1;
+    const bool tw = d->tc_layout == 1, wide = d->KA > hmma::KA_NARROW;
     if (d->tc_layout != 0 && !tw) return set_last_error(1, "maz_infer_recurrent: unknown tc_layout");
     if (tw && (d->o_oh_in <= 0 || d->o_oh_dyn <= 0 || d->o_oh_rg <= 0 || d->o_oh_rg + d->A * 64 > d->vec_floats))
         return set_last_error(1, "maz_infer_recurrent: tc_layout 1 needs the one-hot weight tables behind vec");
@@ -124,13 +131,15 @@ extern "C" int maz_infer_recurrent(const maz_infer_desc *d, void *stream)
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (maz::pdl_mask() & 1) ? 1 : 0;
-    cudaError_t e = tw ? cudaLaunchKernelEx(&cfg, twin::k_recurrent_inference_twin, *d) : cudaLaunchKernelEx(&cfg, fused::k_recurrent_inference, *d);
+    cudaError_t e = !tw ? cudaLaunchKernelEx(&cfg, fused::k_recurrent_inference, *d)
+                    : wide ? twin::launch_wide(cfg, *d)
+                           : cudaLaunchKernelEx(&cfg, twin::k_recurrent_inference_twin<false>, *d);
     if (e != cudaSuccess) return set_last_error(2, std::string("k_recurrent_inference: ") + cudaGetErrorString(e));
     return 0;
 }
 
 // Small-batch variant (infer_hmma.cuh): 32-row tiles on warp-level MMAs.  `d->wpk` / chunk tables must be in the
-// row-major padded layout of mazero_b200/fused.py::HmmaParams.
+// row-major padded layout of mazero_b200/fused.py::HmmaParams.  KA > 48 launches the wide instance.
 extern "C" int maz_infer_small_nq(void) { return hmma::NQ; }
 
 // Opt both kernels into the device's maximum dynamic shared memory, once per device.  (cudaFuncSetAttribute SETS the limit: a
@@ -145,16 +154,15 @@ extern "C" int maz_infer_configure(int vec_floats, int ka)
     if (dev < 0 || dev >= 64 || done[dev]) return 0;
     int optin = 227 * 1024;
     cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    cudaFuncAttributes fa;
-    cudaError_t e = cudaFuncGetAttributes(&fa, hmma::k_recurrent_inference_small);     // (the opt-in limit covers static + dynamic)
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(hmma::k_recurrent_inference_small, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, fused::k_recurrent_inference);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(fused::k_recurrent_inference, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, twin::k_recurrent_inference_twin);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(twin::k_recurrent_inference_twin, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+    const void *kernels[] = {(const void *)hmma::k_recurrent_inference_small<false>, (const void *)hmma::k_recurrent_inference_small<true>,
+                             (const void *)fused::k_recurrent_inference, (const void *)twin::k_recurrent_inference_twin<false>,
+                             twin::wide_kernel()};
+    cudaError_t e = cudaSuccess;
+    for (const void *k : kernels) {
+        cudaFuncAttributes fa;
+        if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, k);     // (the opt-in limit covers static + dynamic)
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+    }
     if (e != cudaSuccess) return set_last_error(2, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e));
     done[dev] = true;
     return 0;
@@ -163,8 +171,9 @@ extern "C" int maz_infer_configure(int vec_floats, int ka)
 extern "C" int maz_infer_recurrent_small(const maz_infer_desc *d, void *stream)
 {
     if (!d) return set_last_error(1, "maz_infer_recurrent_small: NULL descriptor");
-    if (d->B <= 0 || d->N <= 0 || d->N > 32 || d->A <= 0 || d->A > 48 || d->KA % 16 || d->KA < d->A || d->NAP != d->KA)
-        return set_last_error(3, "maz_infer_recurrent_small: unsupported shape (agents <= 32, actions <= 48)");
+    if (d->B <= 0 || d->N <= 0 || d->N > 32 || d->A <= 0 || d->A > hmma::KA_WIDE || d->KA % 16 || d->KA < d->A || d->KA > hmma::KA_WIDE ||
+        d->NAP != d->KA)
+        return set_last_error(3, "maz_infer_recurrent_small: unsupported shape (agents <= 32, actions <= 128)");
     if (!d->pool || !d->actions || !d->next_hidden || !d->reward || !d->value || !d->probs || !d->beta || !d->wpk || !d->vec)
         return set_last_error(1, "maz_infer_recurrent_small: NULL tensor");
     if (d->vec_floats <= 0 || d->vec_floats % 4) return set_last_error(1, "maz_infer_recurrent_small: vec_floats must be a positive multiple of 4");
@@ -188,7 +197,8 @@ extern "C" int maz_infer_recurrent_small(const maz_infer_desc *d, void *stream)
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (maz::pdl_mask() & 1) ? 1 : 0;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, hmma::k_recurrent_inference_small, *d);
+    cudaError_t e = d->KA > hmma::KA_NARROW ? cudaLaunchKernelEx(&cfg, hmma::k_recurrent_inference_small<true>, *d)
+                                            : cudaLaunchKernelEx(&cfg, hmma::k_recurrent_inference_small<false>, *d);
     if (e != cudaSuccess) return set_last_error(2, std::string("k_recurrent_inference_small: ") + cudaGetErrorString(e));
     return 0;
 }

@@ -116,6 +116,8 @@ int maz_search_create(maz_search **out, const maz_search_config *cfg)
         return set_last_error(MAZ_ERR_INVALID, "maz_search_create: dimensions must be positive");
     if (cfg->net_kind == MAZ_NET_SMAC && (!cfg->smac_tc || !cfg->smac_small || cfg->hidden != hmma::H))
         return set_last_error(MAZ_ERR_INVALID, "maz_search_create: MAZ_NET_SMAC needs both weight packings and hidden 128");
+    if (cfg->net_kind == MAZ_NET_SMAC && cfg->A > hmma::KA_WIDE)
+        return set_last_error(MAZ_ERR_UNSUPPORTED, "maz_search_create: the fused SMAC inference supports at most 128 actions per agent");
     if (cfg->net_kind == MAZ_NET_MLP && !cfg->mlp) return set_last_error(MAZ_ERR_INVALID, "maz_search_create: MAZ_NET_MLP needs the MLP descriptor");
     if (cfg->net_kind != MAZ_NET_SMAC && cfg->net_kind != MAZ_NET_MLP) return set_last_error(MAZ_ERR_INVALID, "maz_search_create: bad net_kind");
     int ndev = 0;
@@ -150,9 +152,12 @@ int maz_search_create(maz_search **out, const maz_search_config *cfg)
     // the persistent kernel's shared memory: the inference map + the trees' hot state and the exchange arrays
     int optin = 227 * 1024;
     cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
+    // (the wide instance, KA > 48, places the tree-step scratch that the PH..Q alias cannot hold elsewhere: search_persist.cuh)
+    const bool wide = cfg->net_kind == MAZ_NET_SMAC && s->sm.KA > hmma::KA_NARROW;
     bool persist_ok = cfg->net_kind == MAZ_NET_SMAC && N <= hmma::TM && rpt >= 1 &&
-                      (size_t)rpt * tree_scratch_bytes(s->Nt, A, K, S) <= persist::TREE_SCRATCH_BYTES &&
-                      persist::persist_smem_bytes(s->sm.vec_floats, rpt, s->Nt, A, S) + 256 <= (size_t)optin;
+                      (wide ? persist::persist_smem_bytes_wide(s->sm.vec_floats, rpt, s->Nt, A, K, S) + 256 <= (size_t)optin
+                            : (size_t)rpt * tree_scratch_bytes(s->Nt, A, K, S) <= persist::TREE_SCRATCH_BYTES &&
+                                  persist::persist_smem_bytes(s->sm.vec_floats, rpt, s->Nt, A, S) + 256 <= (size_t)optin);
     if (strat == MAZ_SEARCH_PERSISTENT && !persist_ok) {
         set_last_error(MAZ_ERR_UNSUPPORTED, "maz_search_create: the persistent kernel does not support this network / shape");
         return fail(MAZ_ERR_UNSUPPORTED);
@@ -196,19 +201,20 @@ int maz_search_create(maz_search **out, const maz_search_config *cfg)
         return fail(MAZ_ERR_CUDA);
     }
     if (s->strategy == MAZ_SEARCH_PERSISTENT) {
+        const void *kfn = wide ? (const void *)persist::k_search_persistent<false, true> : (const void *)persist::k_search_persistent<false, false>;
+        const void *kprof = wide ? (const void *)persist::k_search_persistent<true, true> : (const void *)persist::k_search_persistent<true, false>;
         cudaFuncAttributes fa;
-        cudaError_t e = cudaFuncGetAttributes(&fa, persist::k_search_persistent<false>);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(persist::k_search_persistent<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(persist::k_search_persistent<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+        cudaError_t e = cudaFuncGetAttributes(&fa, kfn);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kprof, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
         if (e != cudaSuccess) {
             set_last_error(MAZ_ERR_CUDA, std::string("cudaFuncSetAttribute(k_search_persistent): ") + cudaGetErrorString(e));
             return fail(MAZ_ERR_CUDA);
         }
         int nb = 0;
-        const size_t dyn = persist::persist_smem_bytes(s->sm.vec_floats, rpt, s->Nt, A, S);
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, persist::k_search_persistent<false>, persist::PERSIST_THREADS, dyn);
+        const size_t dyn = wide ? persist::persist_smem_bytes_wide(s->sm.vec_floats, rpt, s->Nt, A, K, S)
+                                : persist::persist_smem_bytes(s->sm.vec_floats, rpt, s->Nt, A, S);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kfn, persist::PERSIST_THREADS, dyn);
         if (e != cudaSuccess || nb < 1) {
             set_last_error(MAZ_ERR_CUDA, "k_search_persistent does not fit on an SM: " + std::to_string(fa.numRegs) + " registers x " +
                                              std::to_string(persist::PERSIST_THREADS) + " threads, " + std::to_string(dyn) + " + " +
@@ -438,9 +444,16 @@ static int launch_persistent(maz_search *s, const maz_search_call *c, bool recor
     if (record) { P.rec_r = s->rec_r; P.rec_v = s->rec_v; P.rec_p = s->rec_p; P.rec_b = s->rec_b; P.rec_ix = s->rec_ix; P.rec_act = s->rec_act; }
     P.tree_clock = s->dbg_clock;
     const unsigned grid = (unsigned)((B + s->rpt - 1) / s->rpt);
-    const size_t dyn = persist::persist_smem_bytes(s->sm.vec_floats, s->rpt, s->Nt, s->cfg.A, s->cfg.S);
-    if (P.tree_clock != nullptr) persist::k_search_persistent<true><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
-    else persist::k_search_persistent<false><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
+    const bool wide = d.KA > hmma::KA_NARROW;
+    const size_t dyn = wide ? persist::persist_smem_bytes_wide(s->sm.vec_floats, s->rpt, s->Nt, s->cfg.A, s->cfg.K, s->cfg.S)
+                            : persist::persist_smem_bytes(s->sm.vec_floats, s->rpt, s->Nt, s->cfg.A, s->cfg.S);
+    if (P.tree_clock != nullptr) {
+        if (wide) persist::k_search_persistent<true, true><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
+        else persist::k_search_persistent<true, false><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
+    } else {
+        if (wide) persist::k_search_persistent<false, true><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
+        else persist::k_search_persistent<false, false><<<grid, persist::PERSIST_THREADS, dyn, s->stream>>>(P);
+    }
     CU_TRY(cudaGetLastError());
     return MAZ_OK;
 }

@@ -58,6 +58,16 @@ __device__ __forceinline__ unsigned long long globaltimer_ns()
 // are not: the tree warps write the next simulation's HH / one-hot rows there)
 constexpr uint32_t TREE_SCRATCH_OFF = OFF_PH;
 constexpr uint32_t TREE_SCRATCH_BYTES = OFF_STAT - OFF_PH;
+// The wide instance (W, 48 < KA <= 128) has larger tree-step scratch (it grows with N*A and S): 2c_vs_64zg (N = 2, A = 70, 8 trees per
+// CTA) needs 8 x 4608 bytes at S = 50 and 8 x 6112 at S = 100, more than the alias above holds.  Its trees beyond that take slots in
+// the X + T tiles, idle during the tree step too (the inference's last reads of them precede the barrier that ends it; the next
+// inference writes them after the barrier that ends the tree step), and then behind the extra map below.
+constexpr uint32_t TREE_SCRATCH_XT_BYTES = OFF_HH - OFF_X;
+__host__ __device__ inline size_t tree_scratch_tail_bytes(int rpt, size_t ts)
+{
+    const int n = rpt - (int)(TREE_SCRATCH_BYTES / ts) - (int)(TREE_SCRATCH_XT_BYTES / ts);
+    return n > 0 ? (size_t)n * ts : 0;
+}
 
 // ---- the CTA's extra shared memory, after the inference kernel's map --------------------------------------------------------
 struct ExtraMap {
@@ -91,9 +101,16 @@ __host__ __device__ inline size_t persist_smem_bytes(int vec_floats, int rpt, in
 {
     return ((smem_bytes(vec_floats) + 15) & ~(size_t)15) + extra_map(rpt, Nt, A, S).bytes;
 }
+// ... of the wide instance: + the tree-step scratch slots behind the extra map
+__host__ __device__ inline size_t persist_smem_bytes_wide(int vec_floats, int rpt, int Nt, int A, int K, int S)
+{
+    return persist_smem_bytes(vec_floats, rpt, Nt, A, S) + tree_scratch_tail_bytes(rpt, tree_scratch_bytes(Nt, A, K, S));
+}
 
 // The parent hidden state and the joint action of ONE root -> its rows of the HH / one-hot tiles (what stage_gather does for the
 // whole tile in the one-step kernel), by the warp that has just selected that root's leaf.  mcts_sampled.py:116-147.
+// W (wide variant): the one-hot tile region holds the row's action instead of its one-hot row.
+template <bool W>
 __device__ __forceinline__ void gather_root(const Desc &d, int root, int rl, int ix, const int *tree_act, int lane)
 {
     HSM_DECL;
@@ -119,7 +136,9 @@ __device__ __forceinline__ void gather_root(const Desc &d, int root, int rl, int
             if (j < N) {
                 const int r = rl * N + j;
                 *reinterpret_cast<uint2 *>(hsm + OFF_HH + (size_t)r * LDA + lane * 8) = make_uint2(pack2(v[u].x, v[u].y), pack2(v[u].z, v[u].w));
-                if (2 * lane < d.KA)
+                if (W) {
+                    if (lane == 0) *reinterpret_cast<int *>(hsm + OFF_ONE + (size_t)r * 4) = act[u];
+                } else if (2 * lane < d.KA)
                     *reinterpret_cast<uint32_t *>(hsm + OFF_ONE + (size_t)r * LDO + lane * 4) =
                         pack2((2 * lane == act[u]) ? 1.f : 0.f, (2 * lane + 1 == act[u]) ? 1.f : 0.f);
             }
@@ -134,8 +153,9 @@ __device__ __forceinline__ void gather_root(const Desc &d, int root, int rl, int
 constexpr int PERSIST_THREADS = NCONS + 128;
 constexpr int REGS_COMPUTE = 232, REGS_PRODUCER = 40;
 
-// kProf: the instance with the in-kernel cycle counters (P.tree_clock); the production instance carries none of their registers
-template <bool kProf>
+// kProf: the instance with the in-kernel cycle counters (P.tree_clock); the production instance carries none of their registers.
+// W: the wide variant of the inference stages (48 < KA <= 128, infer_hmma.cuh).
+template <bool kProf, bool W>
 __global__ void __launch_bounds__(PERSIST_THREADS, 1) k_search_persistent(const __grid_constant__ SearchParams P)
 {
     HSM_DECL;
@@ -149,9 +169,11 @@ __global__ void __launch_bounds__(PERSIST_THREADS, 1) k_search_persistent(const 
         mbar_fence_init();
     }
     setup_rows(d);
-    // the HH / one-hot tiles: rows of roots this CTA does not have stay zero for the whole search
-    for (uint32_t o = tid * 16u; o < TM * (uint32_t)LDA + TM * (uint32_t)LDO; o += PERSIST_THREADS * 16u)
-        *reinterpret_cast<uint4 *>(hsm + OFF_HH + o) = make_uint4(0u, 0u, 0u, 0u);
+    // the HH / one-hot tiles: rows of roots this CTA does not have stay zero (wide variant: action -1) for the whole search
+    for (uint32_t o = tid * 16u; o < TM * (uint32_t)LDA + TM * (uint32_t)LDO; o += PERSIST_THREADS * 16u) {
+        const uint32_t f = (W && o >= TM * (uint32_t)LDA) ? 0xffffffffu : 0u;
+        *reinterpret_cast<uint4 *>(hsm + OFF_HH + o) = make_uint4(f, f, f, f);
+    }
     __syncthreads();
     if (warp >= NCONS / 32) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_PRODUCER));
@@ -172,7 +194,14 @@ __global__ void __launch_bounds__(PERSIST_THREADS, 1) k_search_persistent(const 
     const bool has_tree = warp < rpt && tree < d.B;
     char *tb = P.arena + (size_t)(has_tree ? tree : 0) * L.slab_bytes;
     const size_t B = (size_t)d.B, NA = (size_t)L.N * L.A;
-    const StepScratch scr = carve_step_scratch(reinterpret_cast<char *>(hsm) + TREE_SCRATCH_OFF + (size_t)warp * tree_scratch_bytes(L.N, L.A, L.K, L.S),
+    const size_t ts = tree_scratch_bytes(L.N, L.A, L.K, L.S);
+    char *const base = reinterpret_cast<char *>(hsm);
+    // (wide instance: slots in the PH..Q alias, then in the X + T tiles, then behind the extra map)
+    const int n0 = W ? (int)(TREE_SCRATCH_BYTES / ts) : rpt, n1 = W ? n0 + (int)(TREE_SCRATCH_XT_BYTES / ts) : rpt;
+    const size_t tail0 = ((smem_bytes(d.vec_floats) + 15) & ~(size_t)15) + (W ? extra_map(rpt, L.N, L.A, L.S).bytes : 0);
+    const StepScratch scr = carve_step_scratch(!W || warp < n0 ? base + TREE_SCRATCH_OFF + (size_t)warp * ts
+                                               : warp < n1     ? base + OFF_X + (size_t)(warp - n0) * ts
+                                                               : base + tail0 + (size_t)(warp - n1) * ts,
                                                L.N, L.A, L.K, L.S);
     // ---- shared-memory residents: this warp's tree (header + hot arrays) and the CTA's exchange arrays ------------------------
     const ExtraMap xm = extra_map(rpt, L.N, L.A, L.S);
@@ -249,7 +278,7 @@ __global__ void __launch_bounds__(PERSIST_THREADS, 1) k_search_persistent(const 
                     if (lane == 0) P.rec_ix[o] = ix;
                     for (int j = lane; j < L.N; j += 32) P.rec_act[o * L.N + j] = x_a[warp * L.N + j];
                 }
-                gather_root(d, tree, warp, ix, x_a + warp * L.N, lane);
+                gather_root<W>(d, tree, warp, ix, x_a + warp * L.N, lane);
             }
             if (tree_clk) {
                 const long long q2 = clock64();
@@ -269,7 +298,7 @@ __global__ void __launch_bounds__(PERSIST_THREADS, 1) k_search_persistent(const 
         // profiling: stage timestamps of CTA 0 in the middle simulation, after the per-CTA counters (64 entries)
         long long *sclk = (clk && s == P.S / 2) ? P.tree_clock + 2 * P.S + 4 * (long long)gridDim.x : nullptr;
         if (sclk) { sclk[0] = t2; sclk[1] = t2; }
-        infer_stages(d, io, ring, sclk);
+        infer_stages<W>(d, io, ring, sclk);
         cta_sync();                  // the tile's network outputs are visible to the tree warps; the scratch tiles are free
         if (cta_clk) {
             const long long t3 = clock64();

@@ -11,6 +11,8 @@ import torch
 from ._lib import check, lib
 
 NCHUNK = 32
+A_MAX = 128       # actions per agent of the fused kernels: the wide instances above A_NARROW (csrc/infer_hmma.cuh, csrc/infer_twin.cuh)
+A_NARROW = 48     # ... and of the first-generation tcgen05 kernel (csrc/infer_fused.cuh)
 SWIZZLE = False   # must match MAZ_SWIZZLE in csrc/umma.cuh (128-byte swizzled operand tiles; measured slower)
 H, GH, PH, SUP = 128, 64, 32, 11
 
@@ -85,7 +87,7 @@ def _padrows(w, r):
 def supported(sd, num_agents, action_space_size, hidden):
     d = "dynamics_network."
     try:
-        return (hidden == H and num_agents <= 30 and action_space_size <= 48   # 30 = positional table (attention.py:35)
+        return (hidden == H and num_agents <= 30 and action_space_size <= A_MAX   # 30 = positional table (attention.py:35)
                 and f"{d}attention_stack.2.encoder.layers.2.linear1.weight" in sd
                 and f"{d}attention_stack.2.encoder.layers.3.linear1.weight" not in sd
                 and sd[f"{d}attention_stack.2.encoder.layers.0.linear1.weight"].shape == (H, H)
@@ -241,7 +243,9 @@ class FusedParams:
         dsc.factor, dsc.greedy_pool, dsc.roots_per_tile = ptr(factor), ptr(greedy_pool), int(roots_per_tile)
         import os as _os
         dsc.dbg_flags = int(_os.environ.get('MAZ_DBG_FLAGS', '0'))
-        twin = (not small) and (use_twin(B, self.N) if twin is None else bool(twin))
+        if twin is not None and not twin and not small and self.A > A_NARROW:
+            raise ValueError(f"the first-generation tcgen05 kernel supports at most {A_NARROW} actions per agent (this network has {self.A})")
+        twin = (not small) and (use_twin(B, self.N, self.A) if twin is None else bool(twin))
         dsc.wpk, dsc.vec, dsc.vec_floats = (self.wpk_h if small else self.wpk).data_ptr(), self.vec.data_ptr(), self.vec.numel()
         co, cb = (self.chunk_off_h, self.chunk_bytes_h) if small else (self.chunk_off, self.chunk_bytes)
         if twin:
@@ -271,13 +275,19 @@ FusedParams.weights_desc = _weights_desc
 SMALL_MAX_TILES = int(os.environ.get("MAZ_INFER_SMALL_MAX_TILES", "222"))   # 1.5 waves of 148 SMs (measured cross-over, profiles/prof_infer_cmp.py)
 
 
-def use_twin(B=None, N=None):
+def use_twin(B=None, N=None, A=None):
     """Which large-batch kernel: two tiles in flight per CTA (csrc/infer_twin.cuh) or the first generation, one tile per CTA
-    (csrc/infer_fused.cuh).  MAZ_INFER_TC=twin|v1 forces one.  Cost model from profiles/r02_infer_cmp.log (per launch, B200): a wave
+    (csrc/infer_fused.cuh).  MAZ_INFER_TC=twin|v1 forces one.  With more than A_NARROW actions per agent (A given) only the twin
+    kernel has a (wide) instance: the answer is True, and MAZ_INFER_TC=v1 raises ValueError.  Cost model from profiles/r02_infer_cmp.log (per launch, B200): a wave
     of tile PAIRS takes ~141-146 us whatever the team size, a wave of single first-generation tiles 88 us (N = 3), 96 (N = 5),
     117 (N = 10), 166 (N = 27) ~ 80 + 3.2 N; the kernel with the shorter sum of waves on 148 SMs is taken (e.g. 3m-shaped 16 384
     roots: 3 x 88 us of single tiles beat 2 x 141 us of pairs; 2s3z 4096 roots: one wave of pairs beats two of single tiles)."""
     mode = os.environ.get("MAZ_INFER_TC", "auto")
+    if A is not None and int(A) > A_NARROW:
+        if mode == "v1":
+            raise ValueError(f"MAZ_INFER_TC=v1: the first-generation tcgen05 kernel supports at most {A_NARROW} actions per agent "
+                             f"(this network has {int(A)}); unset MAZ_INFER_TC or set it to twin")
+        return True
     if mode in ("twin", "v1"):
         return mode == "twin"
     if B is None or N is None:

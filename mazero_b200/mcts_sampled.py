@@ -620,7 +620,7 @@ class SampledMCTS(object):
                     import warnings
 
                     warnings.warn("mazero_b200: this network is not the reference SMAC architecture (hidden 128, 3 x 8-head encoder "
-                                  "layers, support 11, <= 30 agents, <= 48 actions): the search runs its forward as plain fp32 torch "
+                                  "layers, support 11, <= 30 agents, <= 128 actions): the search runs its forward as plain fp32 torch "
                                   "ops on the device (parity mode), not through the fused tensor-core kernels", RuntimeWarning,
                                   stacklevel=3)
             inf = SmacInference.from_model(model, device=dev, mode=mode)

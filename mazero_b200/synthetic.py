@@ -17,6 +17,7 @@ WORKLOADS = {
     "2s3z": (5, 11, 4096, 100, 10),
     "mmm2": (10, 18, 8192, 50, 10),
     "27m": (27, 36, 16384, 50, 10),
+    "2c_vs_64zg": (2, 70, 1024, 50, 10),      # 6 + 64 actions per agent: the wide instances of the fused kernels
 }
 
 
