@@ -723,6 +723,7 @@ static __device__ __noinline__ void epi_policy_out(const Desc &d, uint32_t trow,
                 bo[cc + i] = (unit_tau ? v[i] * invs : __powf(v[i], d.inv_tau) * invb);
             }
     }
+    named_bar_sync(1 + t.quad, 128);   // every warp of the quadrant has read `ex`: the next tile's call may overwrite it
 }
 
 // W: the wide variant (48 < NAP <= 128), which differs in the policy output epilogue only (epi_policy_out)

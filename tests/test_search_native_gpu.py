@@ -203,18 +203,19 @@ def test_plan_cache_respects_its_byte_budget(built_lib):
         ms.clear_caches()
 
 
-@pytest.mark.parametrize("gen", ["twin", "v1"])
-@pytest.mark.parametrize("cur", [None, 0, 2])
-def test_graph_loop_on_the_tcgen05_kernels_equals_the_legacy_loop(built_lib, monkeypatch, gen, cur):
+@pytest.mark.parametrize("N,A,gen,cur", [pytest.param(3, 9, g, c, id=f"{c}-{g}") for c in (None, 0, 2) for g in ("twin", "v1")] +
+                         [pytest.param(2, 70, "twin", c, id=f"{c}-twin-A70") for c in (None, 0, 1)])
+def test_graph_loop_on_the_tcgen05_kernels_equals_the_legacy_loop(built_lib, monkeypatch, N, A, gen, cur):
     """The library-built graph with the 128-row tcgen05 kernels (both generations; forced: at this batch size the small-batch
     kernel would be picked) against the round-1 Python loop on the same kernel: in the sequential-agent mode the former assembles
     the joint action INSIDE the inference kernel (factor | tree action | greedy of the parent, mcts_sampled.py:116-147), the latter
-    in Python -- bit-identical SearchOutputs prove the in-kernel assembly of either generation."""
+    in Python -- bit-identical SearchOutputs prove the in-kernel assembly of either generation, and of the wide twin instance
+    (70 actions: only the twin kernel has one)."""
     from mazero_b200.mcts_sampled import SampledMCTS, clear_caches
 
     monkeypatch.setenv("MAZ_INFER_KERNEL", "tcgen05")
     monkeypatch.setenv("MAZ_INFER_TC", gen)
-    N, A, B, K, S = 3, 9, 100, 10, 20
+    B, K, S = 100, 10, 20
     inf, out0, factor, legal = _problem(N, A, B, seed=3)
     cfg = MockConfig(N, A, S, K)
     outs = {}

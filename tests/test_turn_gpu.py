@@ -41,6 +41,12 @@ def test_root_prepare_kernel_matches_numpy_block(built_lib, cur, with_legal, tau
     legal[..., 1] = 1
     Nt = N if cur is None else 1
     noises = rng.dirichlet([0.3] * A, B * Nt).astype(np.float32).reshape(B, Nt, A)
+    if A == 200:   # every row's maximum twice, the copy before or after it: the greedy action is the first one (np.argmax)
+        rows = logits.reshape(B * N, A)
+        first = rows.argmax(-1)
+        other = (first + rng.randint(1, A, size=B * N)) % A
+        rows[np.arange(B * N), other] = rows[np.arange(B * N), first]
+        assert np.array_equal(rows.argmax(-1), np.minimum(first, other)) and (other < first).any() and (other > first).any()
     p_ref, b_ref, n_ref = root_prepare(logits, cur, legal.astype(np.float64) if with_legal else None, noises, 0.25, tau)
     d = lambda x: torch.from_numpy(x).to(DEV)
     dl, dm, dn = d(logits), d(legal), d(noises)

@@ -138,3 +138,67 @@ def test_launch_entries_reject_unsupported_action_counts(built_lib):
     # inside the limits the shape passes and the (NULL) buffers are what is refused
     assert lib.maz_infer_recurrent(ctypes.byref(_desc(2, 70, 1)), None) == _lib.MAZ_ERR_INVALID
     assert lib.maz_infer_recurrent_small(ctypes.byref(_desc(2, 128, 0)), None) == _lib.MAZ_ERR_INVALID
+
+
+def persist_layout(vec_floats, rpt, Nt, A, S, K=10):
+    """The wide persistent kernel's shared memory restated (csrc/search_persist.cuh: persist_smem_bytes_wide, and the placement
+    of each compute warp's tree-step scratch in k_search_persistent): (bytes, trees in the PH..Q alias, trees in the X + T
+    tiles, trees behind the extra map)."""
+    al16 = lambda x: (x + 15) // 16 * 16
+    lv, na = S + 2, Nt * A
+    ts = al16(al16(16 * na + 256 + 4 * 128 + K * Nt) + 24 * lv + 4 * lv + al16(2 * lv))   # tree_scratch_bytes
+    n_alias = min(rpt, 27648 // ts)                      # TREE_SCRATCH_BYTES = OFF_STAT - OFF_PH
+    n_xt = min(rpt - n_alias, 17408 // ts)               # TREE_SCRATCH_XT_BYTES = OFF_HH - OFF_X
+    n_tail = rpt - n_alias - n_xt
+    TM, LDA, LDO, LDP, LDQ, NQ, SUP, LDV = 32, 272, 112, 80, 784, 4, 11, 68
+    off_row = TM * LDA * 3 + TM * LDO + TM * LDP + TM * LDQ + 3 * TM * NQ * 8 + 2 * SUP * LDV * 4
+    off_p = (off_row + TM * 16 + 127) // 128 * 128 + 3 * 128 * 136 * 2
+    hot = 64 + al16(4 * lv) + 3 * al16(2 * lv)
+    extra = hot * rpt + 3 * al16(4 * rpt) + 2 * al16(4 * rpt * na) + al16(4 * rpt * Nt)
+    return al16(off_p + vec_floats * 4 + 128) + extra + n_tail * ts, n_alias, n_xt, n_tail
+
+
+# Every placement of the wide persistent kernel's tree-step scratch, run by tests/test_wide_actions_gpu.py against the legacy loop:
+# name: (N, A, cur (None: joint), S, roots per CTA, B, (alias, X + T, tail), shared-memory bytes).  B None: the handle must be
+# refused (maz_search_create requires bytes + 256 within the opt-in limit: 232 192 bytes on a B200); rpt below min(8, 32 // N)
+# is set with MAZ_SEARCH_RPT.  R1 and P2 sit on the two sides of that limit.
+OPTIN_B200 = 227 * 1024
+PERSIST_CASES = {
+    "P1": (2, 70, None, 50, 8, 45, (6, 2, 0), 214496),
+    "P2": (2, 70, None, 100, 8, 47, (4, 2, 2), 230688),    # the last CTA holds its first tail tree, not its second
+    "P3": (2, 128, 1, 100, 8, 45, (4, 2, 2), 229664),
+    "P4": (2, 128, None, 25, 8, 45, (4, 3, 1), 225920),
+    "P5": (4, 70, None, 12, 8, 37, (4, 3, 1), 227200),
+    "P6": (8, 100, None, 25, 2, 13, (1, 1, 0), 217360),
+    "R1": (2, 128, None, 50, 8, None, (4, 2, 2), 235040),
+    "R2": (8, 100, None, 25, 4, None, (1, 1, 2), 259920),
+}
+
+
+@pytest.mark.parametrize("name", sorted(PERSIST_CASES))
+def test_persist_case_table_matches_the_restated_layout(built_lib, name):
+    N, A, cur, S, rpt, B, counts, nbytes = PERSIST_CASES[name]
+    vec = fused.FusedParams(exact_state_dict(N, A, seed=0), N, A, "cpu").vec.numel()
+    got = persist_layout(vec, rpt, N if cur is None else 1, A, S)
+    assert got == (nbytes, *counts)
+    assert (nbytes + 256 <= OPTIN_B200) == (B is not None)
+
+
+def _cta_placements(case):
+    """(trees in the alias, in the X + T tiles, behind the extra map) of a full CTA and of the last, ragged one"""
+    *_, rpt, B, (n_alias, n_xt, _), _ = case
+    split = lambda r: (min(r, n_alias), min(max(r - n_alias, 0), n_xt), max(r - n_alias - n_xt, 0))
+    return split(rpt), split(B % rpt or rpt)
+
+
+def test_persist_cases_cover_every_placement():
+    """A later change of tree_scratch_bytes or of the case table must not quietly stop running a placement."""
+    run = {k: c for k, c in PERSIST_CASES.items() if c[5] is not None}
+    ctas = [p for c in run.values() for p in _cta_placements(c)]
+    assert any(x == 0 and t == 0 for _, x, t in ctas)                   # trees in the alias only
+    assert any(x > 0 for _, x, _ in ctas)                               # trees in the X + T tiles
+    assert any(t > 0 for _, _, t in ctas)                               # trees behind the extra map
+    assert any(c[2] is not None for c in run.values())                  # a sequential-agent tree
+    assert all(c[5] % c[4] for c in run.values())                       # the last CTA of every case is ragged
+    # P2: the last CTA (47 = 5 x 8 + 7 roots) has its first tail tree and lacks its second
+    assert _cta_placements(run["P2"]) == ((4, 2, 2), (4, 2, 1))

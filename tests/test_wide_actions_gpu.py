@@ -6,7 +6,13 @@
 2. the persistent kernel fits the 2c_vs_64zg shape, and the persistent, graph and legacy loops agree bit for bit at (2, 70);
    the device path replays bit for bit through the CPU oracle tree;
 3. the device-resident environment step (`search_agents`) equals the workers' host loop at (2, 70);
-4. a bf16 search against an fp32 search at 2c_vs_64zg 1024 roots x 50 simulations."""
+4. a bf16 search against an fp32 search at 2c_vs_64zg 1024 roots x 50 simulations;
+5. exact ties of two policy rows: every kernel takes the first of the tied columns (np.argmax), joint and sequential mode;
+6. every placement of the persistent wide kernel's tree-step scratch (the PH..Q alias, the X + T tiles, behind the extra map;
+   tests/test_wide_actions_cpu.py: PERSIST_CASES) against the legacy loop, bit for bit; above the shared-memory limit the
+   persistent strategy is refused and "auto" takes the graph loop."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -15,6 +21,7 @@ from _mock import MockConfig
 from test_infer128_gpu import TOL_BF16, _relerr
 from test_search_gpu import device_path_replay, root_output, smac_model
 from test_search_native_gpu import _equal, _problem
+from test_wide_actions_cpu import OPTIN_B200, PERSIST_CASES, persist_layout
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -91,21 +98,6 @@ def test_first_generation_kernel_refused_above_48_actions(built_lib, monkeypatch
         inf.recurrent_fused(*args)
 
 
-def _persist_smem_bytes(vec_floats, rpt, Nt, A, S, K=10):
-    """persist::persist_smem_bytes_wide (csrc/search_persist.cuh) restated, for the report."""
-    al16 = lambda x: (x + 15) // 16 * 16
-    lv, na = S + 2, Nt * A
-    ts = al16(al16(16 * na + 256 + 4 * 128 + K * Nt) + 24 * lv + 4 * lv + al16(2 * lv))   # tree_scratch_bytes
-    tail = max(0, rpt - 27648 // ts - 17408 // ts) * ts
-    TM, LDA, LDO, LDP, LDQ, NQ, SUP, LDV = 32, 272, 112, 80, 784, 4, 11, 68
-    off_row = TM * LDA * 3 + TM * LDO + TM * LDP + TM * LDQ + 3 * TM * NQ * 8 + 2 * SUP * LDV * 4
-    off_p = (off_row + TM * 16 + 127) // 128 * 128 + 3 * 128 * 136 * 2
-    lv = S + 2
-    hot = 64 + al16(4 * lv) + 3 * al16(2 * lv)
-    extra = hot * rpt + 3 * al16(4 * rpt) + 2 * al16(4 * rpt * Nt * A) + al16(4 * rpt * Nt)
-    return al16(off_p + vec_floats * 4 + 128) + extra + tail
-
-
 @pytest.mark.parametrize("S", [50, 100])
 @pytest.mark.parametrize("joint", [True, False], ids=["joint", "seq"])
 def test_persistent_kernel_fits_2c_vs_64zg(built_lib, joint, S):
@@ -117,8 +109,9 @@ def test_persistent_kernel_fits_2c_vs_64zg(built_lib, joint, S):
     inf = SmacInference(exact_state_dict(N, A, seed=0), N, A, device=DEV, mode="bf16")
     ns = NativeSearch(inf, B, K, S, joint, strategy="persistent")      # maz_search_create refuses when persist_ok fails
     assert ns.strategy == "persistent"
-    smem = _persist_smem_bytes(inf.fused.vec.numel(), 8, N if joint else 1, A, S)
-    print(f"2c_vs_64zg {'joint' if joint else 'seq'} S={S}: persistent kernel shared memory {smem} bytes ({smem / 1024:.1f} KB)")
+    smem, *where = persist_layout(inf.fused.vec.numel(), 8, N if joint else 1, A, S)
+    print(f"2c_vs_64zg {'joint' if joint else 'seq'} S={S}: persistent kernel shared memory {smem} bytes ({smem / 1024:.1f} KB), "
+          f"tree scratch alias / X + T / tail {where}")
     del ns
 
 
@@ -140,17 +133,20 @@ def test_loops_agree_bit_for_bit_at_70_actions(built_lib, cur):
             assert plan.native is None
     clear_caches()
     Nt = N if cur is None else 1
-    print(f"(2, 70) cur={cur}: persistent kernel shared memory {_persist_smem_bytes(inf.fused.vec.numel(), 8, Nt, A, S)} bytes")
+    print(f"(2, 70) cur={cur}: persistent kernel shared memory, tree scratch alias / X + T / tail "
+          f"{persist_layout(inf.fused.vec.numel(), 8, Nt, A, S)}")
     _equal(outs["persistent"], outs["legacy"], "persistent vs legacy: ")
     _equal(outs["graph"], outs["legacy"], "graph vs legacy: ")
     assert int(outs["persistent"].marginal_visit_count[0, 0].sum()) == S
 
 
-@pytest.mark.parametrize("cur", [None, 1])
-def test_device_path_replays_through_oracle_tree_at_70_actions(built_lib, oracle_built, cur):
+# P2 (joint, S = 100): two trees per CTA behind the extra map, the last CTA with only the first of them
+@pytest.mark.parametrize("cur,B,S", [pytest.param(None, 48, 25, id="None"), pytest.param(1, 48, 25, id="1"),
+                                     pytest.param(None, PERSIST_CASES["P2"][5], PERSIST_CASES["P2"][3], id="None-P2")])
+def test_device_path_replays_through_oracle_tree_at_70_actions(built_lib, oracle_built, cur, B, S):
     from mazero_b200.inference import SmacInference
 
-    N, A, B, K, S = 2, 70, 48, 10, 25
+    N, A, K = 2, 70, 10
     model = smac_model(N, A)
     inf = SmacInference.from_model(model, device=DEV, mode="bf16")
     out0 = root_output(model, B)
@@ -232,3 +228,78 @@ def test_bf16_vs_fp32_search_report_2c_vs_64zg(built_lib):
     assert same_sets == 1.0
     assert dv.mean() < 0.02 * max(1.0, np.abs(f.value).max())
     assert tv.mean() < 0.15
+
+
+TIES = ([(40, k, p) for k in ("twin", "tcgen05", "small") for p in ((3, 11), (15, 16), (7, 39))] +
+        [(A, k, p) for A in (70, 128) for k in ("twin", "small") for p in ((5, 21), (31, 32), (2, 67), (1, A - 1))])
+
+
+@pytest.mark.parametrize("A,kernel,pair", TIES, ids=[f"A{a}-{k}-{p[0]}-{p[1]}" for a, k, p in TIES])
+def test_exact_ties_take_the_first_maximum(built_lib, A, kernel, pair):
+    """fc_policy.3 rows and biases j1 < j2 made equal, + 20 on both biases: the two columns tie as the maximum of every row.
+    The kernels reduce across 16-column blocks, 32-column parts (twin) and 8 lanes per row (small-batch); each must keep the
+    first maximum, j1, as np.argmax does (mcts_sampled.py:145), and give both columns the same probability and beta."""
+    from mazero_b200.inference import SmacInference
+    from mazero_b200.synthetic import exact_state_dict
+
+    N, B = 2, 301
+    j1, j2 = pair
+    sd = {k: v.clone() for k, v in exact_state_dict(N, A, seed=A).items()}
+    w, b = sd["prediction_network.fc_policy.3.weight"], sd["prediction_network.fc_policy.3.bias"]
+    w[j2], b[j2] = w[j1], b[j1]
+    b[[j1, j2]] += 20.0
+    inf = SmacInference(sd, N, A, device=DEV, mode="bf16")
+    pool = torch.stack([_hidden(B, N, seed=A), torch.zeros(B, N * 128, device=DEV)])
+    idx = torch.zeros(B, dtype=torch.int32, device=DEV)
+    act = torch.from_numpy(np.random.RandomState(A).randint(0, A, size=(B, N)).astype(np.int32)).to(DEV)
+    for cur in (None, N - 1):
+        Nt = N if cur is None else 1
+        probs, beta, logits = (torch.full((B, n, A), float("nan"), device=DEV) for n in (Nt, Nt, N))
+        greedy = torch.full((B, N), -1, dtype=torch.int32, device=DEV)
+        mode = dict(tree_agents=1, cur=cur, inv_tau=0.5) if cur is not None else {}
+        inf.recurrent_fused(B, pool, idx, act, pool[1], torch.zeros(B, device=DEV), torch.zeros(B, device=DEV), probs, beta, greedy,
+                            logits, kernel=kernel, **mode)
+        torch.cuda.synchronize()
+        what = f"{kernel} A={A} ({j1}, {j2}) {'joint' if cur is None else f'cur={cur}'}"
+        # premise: the tied columns are bit-identical maxima of every row
+        assert torch.equal(logits[..., j1], logits[..., j2]), f"{what}: tied logits differ"
+        assert torch.equal(logits[..., j1], logits.max(-1).values), f"{what}: the tie is not the maximum"
+        assert (greedy == j1).all(), f"{what}: greedy {greedy[greedy != j1][:8].tolist()}"
+        assert torch.equal(probs[..., j1], probs[..., j2]) and torch.equal(beta[..., j1], beta[..., j2]), what
+
+
+@pytest.mark.parametrize("name", sorted(PERSIST_CASES))
+def test_persistent_kernel_every_tree_scratch_placement(built_lib, monkeypatch, name):
+    from mazero_b200.mcts_sampled import SampledMCTS, clear_caches
+    from mazero_b200.search_native import NativeSearch
+
+    N, A, cur, S, rpt, B, counts, nbytes = PERSIST_CASES[name]
+    K = 10
+    if rpt < min(8, 32 // N):
+        monkeypatch.setenv("MAZ_SEARCH_RPT", str(rpt))
+    assert min(8, 32 // N, int(os.environ.get("MAZ_SEARCH_RPT", "8"))) == rpt    # the roots per CTA of maz_search_create
+    inf, out0, factor, legal = _problem(N, A, B or 16)
+    layout = persist_layout(inf.fused.vec.numel(), rpt, N if cur is None else 1, A, S)
+    print(f"{name}: (N, A) = ({N}, {A}) {'joint' if cur is None else f'cur={cur}'} S={S} rpt={rpt} B={B}: {layout[0]} bytes, "
+          f"tree scratch alias / X + T / tail {layout[1:]}")
+    assert layout == (nbytes, *counts)
+    if B is None:
+        assert nbytes + 256 > OPTIN_B200
+        with pytest.raises(RuntimeError, match="persistent kernel does not support"):
+            NativeSearch(inf, 16, K, S, cur is None, strategy="persistent")
+        assert NativeSearch(inf, 16, K, S, cur is None).strategy == "graph"
+        return
+    ns = NativeSearch(inf, B, K, S, cur is None)
+    assert ns.strategy == "persistent"                              # "auto": within the limit, one wave of CTAs
+    del ns
+    cfg = MockConfig(N, A, S, K)
+    outs = {}
+    for strat in ("persistent", "legacy"):
+        mcts = SampledMCTS(cfg, np.random.RandomState(1), search_strategy=strat)
+        outs[strat] = mcts.batch_search(inf, out0, cur, factor, N, legal, DEV, add_noise=True)
+        plan = next(iter(mcts._plans.values()))
+        assert (plan.native.strategy if plan.native is not None else "legacy") == strat
+    clear_caches()
+    _equal(outs["persistent"], outs["legacy"], f"{name}: persistent vs legacy: ")
+    assert int(outs["persistent"].marginal_visit_count[0, 0].sum()) == S
+
