@@ -77,6 +77,39 @@ int maz_infer_small_nq(void);
  * captured into a CUDA graph do not have to); vec_floats / ka as in the descriptor */
 int maz_infer_configure(int vec_floats, int ka);
 
+/* ---- root inference: MAMuZeroNet.initial_inference (config/smac/model.py:542-559) ----------------------------------
+ * representation (config/smac/model.py:176-195: feature_norm LayerNorm over obs_dim, then mlp([obs_dim, 128, 128, 128]))
+ * and the prediction heads (:494-501) + inverse value transform (core/config.py:430-499), one launch of a small-batch tile
+ * kernel (mazero_b200/csrc/infer_initial.cuh): bf16 operands, fp32 accumulate, feature_norm in fp32.  The reward of
+ * initial_inference is zero and is not stored; the policy logits are raw (root preparation, maz_root_prepare_dev, applies the
+ * noise, the legal mask and the softmax).  Device pointers only; asynchronous on the stream, no allocation, no synchronisation.
+ * Errors: MAZ_ERR_INVALID for NULL pointers, B <= 0, N outside 1..30, a malformed parameter vector or chunk table;
+ * MAZ_ERR_UNSUPPORTED for H != 128, A > 128, obs_dim > 640.  The weight packings: see mazero_b200/fused.py. */
+typedef struct maz_initial_desc {
+    int B, N, A, H, obs_dim;     /* roots, agents, actions per agent, hidden per agent (128), observation features per agent */
+    const float *obs;            /* (B*N, obs_dim) fp32, C-contiguous */
+    float *hidden;               /* (B, N*128) root hidden state */
+    float *value;                /* (B,) after the inverse value transform */
+    float *policy_logits;        /* (B, N, A) */
+    /* representation network, kp = obs_dim rounded up to 16:
+     * rep_wpk: bf16 row-major chunks with 8 elements of row padding -- mlp.0.weight (zero columns up to kp) as column blocks of
+     *   <= 128 features, each [128][kc + 8]; then mlp.3.weight and mlp.6.weight, [128][136] each;
+     * rep_vec: fp32 feature_norm.weight, feature_norm.bias (kp each, zero padded), mlp.0.bias, mlp.1.weight, mlp.1.bias,
+     *   mlp.3.bias, mlp.4.weight, mlp.4.bias, mlp.6.bias (128 each) */
+    const void *rep_wpk;
+    const float *rep_vec;
+    /* prediction heads: the small-batch packing of maz_infer_desc (wpk, vec, chunk tables, o_vg, o_pol); the kernel reads
+     * chunks 27, 28, 30, 31 and vec[o_vg, vec_floats) */
+    const void *wpk;
+    const float *vec;
+    int vec_floats;
+    unsigned int chunk_off[MAZ_INFER_NCHUNK];
+    unsigned int chunk_bytes[MAZ_INFER_NCHUNK];
+    int o_vg, o_pol;
+} maz_initial_desc;
+
+int maz_infer_initial(const maz_initial_desc *desc, void *cuda_stream);
+
 /* ---- MLP-family network (the reference's matrix-game MAMuZeroNet) --------------------------------------------
  * Replaces, for the search only, config/matrix/model.py:358-368 `recurrent_inference` (= `dynamics` :334-343 /
  * DynamicsNetwork.forward :118-126 + PredictionNetwork.forward :163-166) and the driver's softmax / beta

@@ -50,6 +50,7 @@ SIGNATURES = {
     "maz_infer_recurrent_small": (C.c_int, [C.c_void_p, C.c_void_p]),
     "maz_infer_small_nq": (C.c_int, []),
     "maz_infer_configure": (C.c_int, [C.c_int, C.c_int]),
+    "maz_infer_initial": (C.c_int, [C.c_void_p, C.c_void_p]),
     "maz_mlp_recurrent": (C.c_int, [C.c_void_p, C.c_void_p]),
     "maz_mlp_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     # include/maz_hostrng.h

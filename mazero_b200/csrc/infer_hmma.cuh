@@ -795,7 +795,8 @@ __device__ __forceinline__ void gnn_phase_c(const Thr &th, uint32_t stat, float 
 
 // heads, first layers, ONE stage: reward GNN layer 1 on [next_hidden | onehot], value GNN layer 1 and fc_policy.0 on
 // next_hidden.  Outputs: X[:, 0:64] = reward features, X[:, 64:128] = value features, Ph = relu(LN(policy hidden)).
-template <bool W>
+// R: the root variant of initial_inference (infer_initial.cuh): no reward head, so its two weight chunks are not consumed.
+template <bool W, bool R = false>
 static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
 {
     const Thr th;
@@ -803,12 +804,15 @@ static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
     const int n0 = CW * th.nq, ldo = (d.KA + PAD) * 2;
     float aR[NT][4], aV[NT][4], aP[2][4];
     zero<NT>(aR); zero<NT>(aV); zero<2>(aP);
-    uint32_t w = ring.acquire();
-    gemm_fixed<NT, 8>(aR, th, sb + OFF_T, LDA, w, LDA, n0);
-    ring.release(th.lane);
-    w = ring.acquire();
-    gemm_action<W, NT>(aR, th, sb, w, ldo, n0, d.KA);
-    ring.release(th.lane);
+    uint32_t w;
+    if constexpr (!R) {
+        w = ring.acquire();
+        gemm_fixed<NT, 8>(aR, th, sb + OFF_T, LDA, w, LDA, n0);
+        ring.release(th.lane);
+        w = ring.acquire();
+        gemm_action<W, NT>(aR, th, sb, w, ldo, n0, d.KA);
+        ring.release(th.lane);
+    }
     w = ring.acquire();
     gemm_fixed<NT, 8>(aV, th, sb + OFF_T, LDA, w, LDA, n0);
     ring.release(th.lane);
@@ -818,7 +822,7 @@ static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
     const uint32_t G = sb + OFF_Q, stat = sb + OFF_STAT, pr = sb + OFF_P + 4u * d.o_rg, pvv = sb + OFF_P + 4u * d.o_vg;
     const uint32_t pp = sb + OFF_P + 4u * d.o_pol;
     // phase A
-    gnn_phase_a(aR, th, G + 4u * G_R, pr);
+    if constexpr (!R) gnn_phase_a(aR, th, G + 4u * G_R, pr);
     gnn_phase_a(aV, th, G + 4u * G_V, pvv);
     if (th.nq < 2) add_bias<2>(aP, th, pp, 16 * th.nq);
     stats_write<2>(aP, th, stat + 2 * STAT_SET);          // (warps nq >= 2 contribute zeros)
@@ -826,7 +830,7 @@ static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
     // phase B
     const int r0A = row_info(th.rA).r0, r0B = row_info(th.rB).r0;
     float yR[GT][4], yV[GT][4];
-    gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, d.N, r0A, r0B, yR);
+    if constexpr (!R) gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, d.N, r0A, r0B, yR);
     gnn_phase_b(aV, th, G + 4u * G_V, pvv, stat + STAT_SET, d.N, r0A, r0B, yV);
     if (th.nq < 2) {                                      // policy hidden: relu(LN(acc + b) * g + be) over 32 columns
         float mA, sA, mB, sB;
@@ -844,9 +848,9 @@ static __device__ __noinline__ void stage_heads1(const Desc &d, Ring &ring)
     }
     cta_sync();
     // phase C
-    gnn_phase_c(th, stat, yR);
+    if constexpr (!R) gnn_phase_c(th, stat, yR);
     gnn_phase_c(th, stat + STAT_SET, yV);
-    store_tile<GT>(sb + OFF_X, LDA, th, FW * th.nq, yR);
+    if constexpr (!R) store_tile<GT>(sb + OFF_X, LDA, th, FW * th.nq, yR);
     store_tile<GT>(sb + OFF_X, LDA, th, GH + FW * th.nq, yV);
     cta_sync();
 }
@@ -942,7 +946,9 @@ __device__ __forceinline__ void policy_outputs(const Desc &d, const SimIo io, ui
 // fc_policy.3 -> softmax / beta / greedy (mcts_sampled.py:158-161).  The narrow variant stages the policy logits in the q|k|v
 // region and computes the policy outputs in phase B; the wide variant keeps its PB logit blocks per warp in registers until
 // phase D has consumed the layer-2 features and then uses the X + T tiles (one more barrier).
-template <bool W>
+// R: the root variant of initial_inference (infer_initial.cuh): no reward head (its weight chunk is not consumed); the policy
+// logits + bias go from the fragments straight to io.logits_out (B, N, A), with no softmax / beta / greedy; value to io.value.
+template <bool W, bool R = false>
 static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, const SimIo io, long long *hs_clk)
 {
     const Thr th;
@@ -958,9 +964,12 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     zero<NT>(aR); zero<NT>(aV);
 #pragma unroll
     for (int bk = 0; bk < PB; ++bk) zero<2>(aP[bk]);
-    uint32_t w = ring.acquire();
-    gemm_fixed<NT, 4>(aR, th, sb + OFF_X, LDA, w, ldg, n0);
-    ring.release(th.lane);
+    uint32_t w;
+    if constexpr (!R) {
+        w = ring.acquire();
+        gemm_fixed<NT, 4>(aR, th, sb + OFF_X, LDA, w, ldg, n0);
+        ring.release(th.lane);
+    }
     w = ring.acquire();
     gemm_fixed<NT, 4>(aV, th, sb + OFF_X + GH * 2, LDA, w, ldg, n0);
     ring.release(th.lane);
@@ -974,9 +983,28 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     const uint32_t PL = G + 4u * PL0;
     HS();
     // phase A
-    gnn_phase_a(aR, th, G + 4u * G_R, pr);
+    if constexpr (!R) gnn_phase_a(aR, th, G + 4u * G_R, pr);
     gnn_phase_a(aV, th, G + 4u * G_V, pvv);
-    if (!W && pc0 < d.NAP) {                                       // policy logits + bias -> fp32 scratch [TM][48]
+    if constexpr (R) {                                             // root logits + bias -> global (B, N, A)
+        const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
+        const RowInfo ra = row_info(th.rA), rb = row_info(th.rB);
+#pragma unroll
+        for (int bk = 0; bk < PB; ++bk) {
+#pragma unroll
+            for (int tl = 0; tl < 2; ++tl) {
+                const int c = pc0 + NQ * 16 * bk + 8 * tl + 2 * th.t;
+                if (c >= d.NAP) continue;
+                const float2 bb = ldp2(b2 + 4u * c);
+#pragma unroll
+                for (int hf = 0; hf < 2; ++hf) {
+                    const RowInfo &ri = hf ? rb : ra;
+                    float *lo = io.logits_out + ((size_t)ri.root * N + ri.agent) * d.A;
+                    if (ri.valid && c < d.A) lo[c] = aP[bk][tl][2 * hf] + bb.x;
+                    if (ri.valid && c + 1 < d.A) lo[c + 1] = aP[bk][tl][2 * hf + 1] + bb.y;
+                }
+            }
+        }
+    } else if (!W && pc0 < d.NAP) {                                       // policy logits + bias -> fp32 scratch [TM][48]
         const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
 #pragma unroll
         for (int tl = 0; tl < 2; ++tl) {
@@ -991,20 +1019,22 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     // phase B
     const int r0A = row_info(th.rA).r0, r0B = row_info(th.rB).r0;
     float yR[GT][4], yV[GT][4];
-    gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, N, r0A, r0B, yR);
+    if constexpr (!R) gnn_phase_b(aR, th, G + 4u * G_R, pr, stat, N, r0A, r0B, yR);
     gnn_phase_b(aV, th, G + 4u * G_V, pvv, stat + STAT_SET, N, r0A, r0B, yV);
     // the raw (post-ReLU) layer-2 features, fp32 -> Y in the X + T tiles (free since the GEMMs above)
     const uint32_t YB = sb + OFF_X;
 #pragma unroll
     for (int tl = 0; tl < GT; ++tl) {
         const int f = FW * th.nq + 8 * tl + 2 * th.t;
-        sts2f(YB + 4u * (Y_R + th.rA * GH + f), yR[tl][0], yR[tl][1]);
-        sts2f(YB + 4u * (Y_R + th.rB * GH + f), yR[tl][2], yR[tl][3]);
+        if constexpr (!R) {
+            sts2f(YB + 4u * (Y_R + th.rA * GH + f), yR[tl][0], yR[tl][1]);
+            sts2f(YB + 4u * (Y_R + th.rB * GH + f), yR[tl][2], yR[tl][3]);
+        }
         sts2f(YB + 4u * (Y_V + th.rA * GH + f), yV[tl][0], yV[tl][1]);
         sts2f(YB + 4u * (Y_V + th.rB * GH + f), yV[tl][2], yV[tl][3]);
     }
     HS();
-    if constexpr (!W) policy_outputs<KA_NARROW>(d, io, PL, hs_clk, hs_n);
+    if constexpr (!W && !R) policy_outputs<KA_NARROW>(d, io, PL, hs_clk, hs_n);
     HS();
     cta_sync();
     HS();
@@ -1014,7 +1044,7 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     const int rpt = tile_rpt(d);
     const uint32_t POOL = G;
     const float invn = 1.f / (float)N;
-    for (int i = tid; i < 2 * rpt * (GH / 2); i += NCONS) {
+    for (int i = (R ? rpt * (GH / 2) : 0) + tid; i < 2 * rpt * (GH / 2); i += NCONS) {   // (R: the value head only)
         const int f2 = i & (GH / 2 - 1), rest = i >> 5, kind = rest >= rpt ? 1 : 0, rl = rest - kind * rpt;
         const uint32_t src = YB + 4u * ((kind ? Y_V : Y_R) + (rl * N) * GH + 2 * f2), st = stat + (kind ? STAT_SET : 0u);
         float2 s = make_float2(0.f, 0.f);
@@ -1040,7 +1070,7 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     }
     cta_sync();
     HS();
-    if constexpr (W) {                                             // the layer-2 features are consumed: logits + bias -> X + T tiles
+    if constexpr (W && !R) {                                       // the layer-2 features are consumed: logits + bias -> X + T tiles
         const uint32_t b2 = sb + OFF_P + 4u * (d.o_pol + 96);
 #pragma unroll
         for (int bk = 0; bk < PB; ++bk) {
@@ -1061,8 +1091,10 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
     // softmax . support -> inv_h and stores the scalar.  No barrier, no shared-memory round trip.
     {
         const int hw = tid >> 4, l16 = tid & 15, lane = tid & 31;
-        for (int pair = hw; pair < rpt * 2; pair += NCONS / 16) {      // (both half-warps of a warp run the same number of rounds)
-            const int rl = pair >> 1, kind = pair & 1;
+        // (both half-warps of a warp run the same number of rounds; R: one value head per half-warp, rounded up to whole warps)
+        const int npair = R ? (rpt + 1) & ~1 : rpt * 2;
+        for (int pair = hw; pair < npair; pair += NCONS / 16) {
+            const int rl = R ? pair : pair >> 1, kind = R ? 1 : pair & 1;
             float logit = 0.f;
             if (l16 < SUP) {
                 const uint32_t pv = POOL + 4u * ((kind * rpt + rl) * GH), vw = sb + OFF_VP + 4u * ((kind * SUP + l16) * LDV);
@@ -1086,11 +1118,11 @@ static __device__ __noinline__ void stage_heads2(const Desc &d, Ring &ring, cons
 #pragma unroll
             for (int k = 0; k < SUP; ++k) v[k] = __shfl_sync(0xffffffffu, logit, (lane & 16) + k);
             const int root = blockIdx.x * rpt + rl;
-            if (l16 == 0 && root < d.B) (kind ? io.value : io.reward)[root - io.root0] = support_to_scalar(v);
+            if (l16 == 0 && root < d.B && (!R || rl < rpt)) (kind ? io.value : io.reward)[root - io.root0] = support_to_scalar(v);
         }
     }
     HS();
-    if constexpr (W) {
+    if constexpr (W && !R) {
         cta_sync();
         policy_outputs<KA_WIDE>(d, io, sb + OFF_X, hs_clk, hs_n);
     }

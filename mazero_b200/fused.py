@@ -32,6 +32,19 @@ class InferDesc(C.Structure):
     ]
 
 
+class InitialDesc(C.Structure):      # include/maz_infer.h: maz_initial_desc
+    _fields_ = [
+        ("B", C.c_int), ("N", C.c_int), ("A", C.c_int), ("H", C.c_int), ("obs_dim", C.c_int),
+        ("obs", C.c_void_p), ("hidden", C.c_void_p), ("value", C.c_void_p), ("policy_logits", C.c_void_p),
+        ("rep_wpk", C.c_void_p), ("rep_vec", C.c_void_p), ("wpk", C.c_void_p), ("vec", C.c_void_p), ("vec_floats", C.c_int),
+        ("chunk_off", C.c_uint * NCHUNK), ("chunk_bytes", C.c_uint * NCHUNK), ("o_vg", C.c_int), ("o_pol", C.c_int),
+    ]
+
+
+OBS_MAX = 640     # observation features per agent of the root-inference kernel (csrc/infer_initial.cuh)
+REP = "representation_network."
+
+
 def _pad16(n):
     return (n + 15) // 16 * 16
 
@@ -102,6 +115,55 @@ def supported(sd, num_agents, action_space_size, hidden):
         return False
 
 
+def supported_initial(sd, num_agents, action_space_size, hidden):
+    """The root-inference kernel (csrc/infer_initial.cuh, `maz_infer_initial`) takes the reference representation network
+    (config/smac/model.py:176-195, use_feature_norm): feature_norm, then mlp([obs, 128, 128, 128]) = Linear, LayerNorm, ReLU,
+    Linear, LayerNorm, ReLU, Linear (mlp.{0,1,3,4,6}), 1 <= obs <= 640, on top of the heads `supported` takes."""
+    return initial_unsupported_reason(sd, num_agents, action_space_size, hidden) is None
+
+
+def initial_unsupported_reason(sd, num_agents, action_space_size, hidden):
+    if not supported(sd, num_agents, action_space_size, hidden):
+        return ("the network is not the reference SMAC architecture the fused kernels take (hidden 128, 3 x 8-head encoder "
+                "layers, support 11, <= 30 agents, <= 128 actions)")
+    m = REP + "mlp."
+    if f"{m}0.weight" not in sd:
+        return "the state dict holds no representation network"
+    if f"{REP}feature_norm.weight" not in sd or f"{REP}feature_norm.bias" not in sd:
+        return "the representation network has no feature_norm (use_feature_norm=False)"
+    layers = sorted(int(k[len(m):].split(".")[0]) for k in sd if k.startswith(m) and k.endswith(".weight"))
+    if layers != [0, 1, 3, 4, 6]:
+        return f"the representation mlp must be Linear, LN, ReLU, Linear, LN, ReLU, Linear (mlp.0/1/3/4/6), not layers {layers}"
+    obs = sd[f"{m}0.weight"].shape[1]
+    shapes = {f"{REP}feature_norm.weight": (obs,), f"{REP}feature_norm.bias": (obs,), f"{m}0.weight": (H, obs), f"{m}0.bias": (H,),
+              f"{m}1.weight": (H,), f"{m}1.bias": (H,), f"{m}3.weight": (H, H), f"{m}3.bias": (H,), f"{m}4.weight": (H,),
+              f"{m}4.bias": (H,), f"{m}6.weight": (H, H), f"{m}6.bias": (H,)}
+    for k, shp in shapes.items():
+        if k not in sd or tuple(sd[k].shape) != shp:
+            return f"representation parameter {k}: expected shape {shp} (widths [obs, 128, 128, 128])"
+    if not 1 <= obs <= OBS_MAX:
+        return f"observation size {obs} outside 1..{OBS_MAX}"
+    return None
+
+
+def pack_representation(sd, device):
+    """The representation network in the layout of maz_initial_desc (include/maz_infer.h): bf16 row-major chunks with 8 elements
+    of padding -- mlp.0 (zero columns up to kp = obs rounded up to 16) as column blocks of <= 128 features, then mlp.3, mlp.6 --
+    and one fp32 vector: feature_norm weight / bias (zero padded to kp), mlp.0 bias, mlp.1 w / b, mlp.3 bias, mlp.4 w / b,
+    mlp.6 bias.  Returns (wpk bf16 flat, vec fp32, obs)."""
+    g = lambda k: sd[REP + k].detach().to(device=device, dtype=torch.float32)
+    w0 = g("mlp.0.weight")
+    obs = w0.shape[1]
+    kp = _pad16(obs)
+    w0 = _padcols(w0, kp)
+    chunks = [w0[:, k0:k0 + 128] for k0 in range(0, kp, 128)] + [g("mlp.3.weight"), g("mlp.6.weight")]
+    wpk = torch.cat([pack_rowmajor(c.contiguous()) for c in chunks])
+    pad = lambda v: torch.cat([v, torch.zeros(kp - obs, device=v.device)])
+    vec = torch.cat([pad(g("feature_norm.weight")), pad(g("feature_norm.bias")), g("mlp.0.bias"), g("mlp.1.weight"),
+                     g("mlp.1.bias"), g("mlp.3.bias"), g("mlp.4.weight"), g("mlp.4.bias"), g("mlp.6.bias")]).contiguous()
+    return wpk, vec, obs
+
+
 class FusedParams:
     """Device-resident packed parameters + the constant half of the launch descriptor."""
 
@@ -111,6 +173,7 @@ class FusedParams:
         self.device = torch.device(device)
         self.wpk = None
         self.vec = None
+        self.rep_wpk = self.rep_vec = None     # representation network (root inference), when the state dict has a supported one
         self.repack(sd)
 
     def repack(self, sd):
@@ -227,6 +290,28 @@ class FusedParams:
             self.wpk.copy_(wpk)
             self.vec.copy_(vecf)
             self.vec_t.copy_(vec_t)
+        if supported_initial(sd, N, A, H):
+            rw, rv, self.obs_dim = pack_representation(sd, dev)
+            if self.rep_wpk is None or self.rep_wpk.shape != rw.shape:
+                self.rep_wpk, self.rep_vec = rw, rv
+            else:
+                self.rep_wpk.copy_(rw)
+                self.rep_vec.copy_(rv)
+
+    def initial_desc(self, B, obs, hidden, value, policy_logits):
+        """maz_initial_desc for `maz_infer_initial`: obs (B*N, obs_dim) fp32, outputs hidden (B, N*128), value (B,),
+        policy_logits (B, N, A); device tensors (or None for a bare descriptor)."""
+        ptr = lambda t: (t.data_ptr() if t is not None else None)
+        dsc = InitialDesc()
+        dsc.B, dsc.N, dsc.A, dsc.H = int(B), self.N, self.A, H
+        dsc.obs_dim = int(self.obs_dim) if self.rep_wpk is not None else 0
+        dsc.obs, dsc.hidden, dsc.value, dsc.policy_logits = ptr(obs), ptr(hidden), ptr(value), ptr(policy_logits)
+        dsc.rep_wpk, dsc.rep_vec = ptr(self.rep_wpk), ptr(self.rep_vec)
+        dsc.wpk, dsc.vec, dsc.vec_floats = self.wpk_h.data_ptr(), self.vec.data_ptr(), self.vec.numel()
+        for i in range(NCHUNK):
+            dsc.chunk_off[i], dsc.chunk_bytes[i] = self.chunk_off_h[i], self.chunk_bytes_h[i]
+        dsc.o_vg, dsc.o_pol = self.off["vg"], self.off["pol"]
+        return dsc
 
     def desc(self, B, pool, idx_x, actions, next_hidden, reward, value, probs, beta, greedy=None, logits_out=None,
              tree_agents=None, cur=-1, inv_tau=1.0, dbg_clock=None, small=False, factor=None, greedy_pool=None, roots_per_tile=0,
@@ -306,6 +391,10 @@ def use_small(B, N):
         return mode == "small"
     rpt = 32 // N
     return (B + rpt - 1) // rpt <= SMALL_MAX_TILES
+
+
+def launch_initial(dsc, stream_ptr):
+    check(lib.maz_infer_initial(C.byref(dsc), C.c_void_p(stream_ptr)))
 
 
 def launch(dsc, stream_ptr, small=False):

@@ -91,6 +91,13 @@ class SmacInference:
             idx += 3
         self.rsup = torch.arange(reward_support[0], reward_support[1] + 1, dtype=torch.float32, device=dev)
         self.vsup = torch.arange(value_support[0], value_support[1] + 1, dtype=torch.float32, device=dev)
+        # representation network (initial_inference): row-wise MLP kernel, when the state dict holds it and a GPU is there.
+        # (Built first: its parameters join the registry that the fused path packs for the root-inference kernel.)
+        self.rep = None
+        if "representation_network.mlp.0.weight" in sd and dev.type == "cuda":
+            from .inference_mlp import RowMlp
+
+            self.rep = RowMlp(sd, dev, self._params)
         # fused tensor-core path (bf16 operands, fp32 accumulate): csrc/infer_fused.cuh
         self.fused = None
         if mode == "bf16":
@@ -103,12 +110,6 @@ class SmacInference:
                 raise RuntimeError("mode='bf16': network shape not supported by the fused kernel "
                                    "(needs the reference SMAC architecture: hidden 128, 3 layers, 8 heads, support 11)")
             self.fused = fused.FusedParams(self._params, self.N, self.A, dev)
-        # representation network (initial_inference): row-wise MLP kernel, when the state dict holds it and a GPU is there
-        self.rep = None
-        if "representation_network.mlp.0.weight" in sd and dev.type == "cuda":
-            from .inference_mlp import RowMlp
-
-            self.rep = RowMlp(sd, dev, self._params)
 
     @classmethod
     def from_model(cls, model, device="cuda", mode="fp32", **kw):
@@ -131,15 +132,40 @@ class SmacInference:
         if self.rep is not None:
             self.rep.retranspose()
 
-    def initial_inference(self, observation):
+    def initial_inference(self, observation, fused=False):
         """`MAMuZeroNet.initial_inference` (config/smac/model.py:542-559) without leaving the device: observation
         (B, N, ...) -> NetworkOutput(hidden (B, N*H), reward zeros (B,1), value (B,1), policy_logits (B,N,A)) as CUDA tensors
-        with no synchronisation (the reference's eval mode does `.cpu().numpy()` on value and logits)."""
+        with no synchronisation (the reference's eval mode does `.cpu().numpy()` on value and logits).
+        fused=False: fp32, the row-wise MLP kernel for the representation and torch ops for the heads.  fused=True: one launch
+        of the bf16 root-inference kernel (csrc/infer_initial.cuh, `maz_infer_initial`); needs mode="bf16" and the reference
+        representation network (`fused.supported_initial`), else ValueError."""
+        from .synthetic import NetworkOutput
+        if fused:
+            return NetworkOutput(*self._initial_fused(observation))
         if self.rep is None:
             raise RuntimeError("the state dict holds no representation network (or no CUDA device)")
         from .inference_mlp import initial_inference_device
-        from .synthetic import NetworkOutput
         return NetworkOutput(*initial_inference_device(self, self.rep, observation))
+
+    def _initial_fused(self, observation, stream=None):
+        from . import fused
+
+        if self.fused is None:
+            raise ValueError(f"initial_inference(fused=True) needs SmacInference(mode='bf16'), this object has mode={self.mode!r}")
+        if self.fused.rep_wpk is None:
+            raise ValueError("initial_inference(fused=True): " + (fused.initial_unsupported_reason(self._params, self.N, self.A, self.H)
+                                                                  or "representation network not packed"))
+        B = observation.shape[0]
+        x = observation.reshape(B * self.N, -1).to(device=self.device, dtype=torch.float32).contiguous()
+        if x.shape[1] != self.fused.obs_dim:
+            raise ValueError(f"initial_inference(fused=True): {x.shape[1]} observation features per agent, the representation "
+                             f"network takes {self.fused.obs_dim}")
+        hidden = torch.empty(B, self.N * self.H, dtype=torch.float32, device=self.device)
+        value = torch.empty(B, 1, dtype=torch.float32, device=self.device)
+        logits = torch.empty(B, self.N, self.A, dtype=torch.float32, device=self.device)
+        dsc = self.fused.initial_desc(B, x, hidden, value, logits)
+        fused.launch_initial(dsc, (stream if stream is not None else torch.cuda.current_stream(self.device)).cuda_stream)
+        return hidden, torch.zeros(B, 1, dtype=torch.float32, device=self.device), value, logits
 
     def recurrent_fused(self, B, pool, idx_x, actions, next_hidden, reward, value, probs, beta, greedy=None,
                         logits_out=None, tree_agents=None, cur=-1, inv_tau=1.0, stream=None, dbg_clock=None, kernel=None):
