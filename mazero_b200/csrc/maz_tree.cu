@@ -102,7 +102,8 @@ static int build_layout(TreeLayout &L, int B, int N, int A, int K, int S, float 
     L.off_vsval = take(4ull * L.L);
     L.off_depth = take(2ull * (S + 4));      // depth of the e-th expanded node (its distance from the root)
     {   // wide selection: worth it once the sequential descent (~2 k cycles per level) costs more than one pass over all expanded
-        // nodes (~4 k cycles per 32 of them).  MAZ_SELECT_WIDE=0 never, 1 always (tests run both: identical results).
+        // nodes (~4 k cycles per 32 of them).  MAZ_SELECT_WIDE=0 never, 1 always: identical results
+        // (the fused-step cases of tests/test_tree_gpu.py and tests/test_deep_trees_gpu.py run all three settings).
         const char *e = getenv("MAZ_SELECT_WIDE");
         const int chunks = (S + 1 + 31) / 32;
         L.wide_min_len = e ? (atoi(e) ? 0 : 1 << 30) : 3 + 2 * chunks;

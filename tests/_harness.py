@@ -96,6 +96,36 @@ def drive(tree, inp, K, sims=None, mcts=MCTS, record_steps=True):
     return out
 
 
+def drive_fused(tree, inp, K, mcts=MCTS):
+    """`drive` in the launch order of the on-device loop (maz_search.cu: enqueue_loop), on torch CUDA copies of the arrays:
+    prepare, the selection of simulation 0, then for s < S-1 the fused expansion + backup of s and selection of s+1 (the
+    two-warp kernel, which holds the wide selection), the last expansion + backup alone, the readouts.  Same dict as `drive`."""
+    import torch
+
+    B, N, S = inp.B, inp.N, inp.S
+    dev = torch.device("cuda:0")
+    d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+    rewards, values, probs, beta = d(inp.rewards), d(inp.values), d(inp.probs), d(inp.beta)
+    ix = torch.empty(S, B, dtype=torch.int32, device=dev)
+    iy = torch.empty(B, dtype=torch.int32, device=dev)
+    act = torch.empty(S, B, N, dtype=torch.int32, device=dev)
+    c_base, c_init, discount = mcts["pb_c_base"], mcts["pb_c_init"], mcts["discount"]
+    tree.prepare(rewards[0], values[0], probs[0], beta[0], K, float(inp.noise_eps), d(inp.noises))
+    if S > 0:
+        tree.batch_selection_device(c_base, c_init, discount, ix[0], iy, act[0])
+    for s in range(S - 1):
+        tree.expansion_backup_selection_device(s + 1, discount, K, rewards[s + 1], values[s + 1], probs[s + 1], beta[s + 1],
+                                               c_base, c_init, ix[s + 1], iy, act[s + 1])
+    if S > 0:
+        tree.batch_expansion_and_backup(S, discount, K, rewards[S], values[S], probs[S], beta[S])
+    tree.check()
+    if S > 0:
+        assert iy.cpu().tolist() == list(range(B))
+    out = {"sel_idx": ix.cpu().numpy(), "sel_act": act.cpu().numpy()}
+    out.update(readouts(tree, discount))
+    return out
+
+
 LIST_FIELDS = ("sampled_actions", "sampled_visit_count", "sampled_pred_probs", "sampled_beta", "sampled_beta_hat",
                "sampled_priors", "sampled_imp_ratio", "sampled_pred_values", "sampled_mcts_values", "sampled_rewards",
                "sampled_qvalues")

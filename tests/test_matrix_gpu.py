@@ -79,7 +79,7 @@ def test_matrix_search_on_device_replays_bit_exact(built_lib, oracle_built, kind
         pol, v = net.prediction(hidden)
         value = net._inv(v, net.value_support)
     out0 = NetworkOutput(hidden.cuda(), np.zeros((B, 1), np.float32), value.numpy().reshape(B, 1), pol.numpy())
-    o = device_path_replay(inf, out0, n, a, B, K, S, cur, oracle_built)
+    o, _ = device_path_replay(inf, out0, n, a, B, K, S, cur, oracle_built)
     assert (o.marginal_visit_count.sum(axis=(1, 2)) == S * (n if cur is None else 1)).all()
 
 

@@ -47,9 +47,10 @@ def test_step_path_reproduces_reference_known_answers(built_lib):
     check_kat(*sequential_search(fn, cfg, model, legal=kat_legal()))
 
 
-def device_path_replay(inf, out0, N, A, B, K, S, cur, oracle_built):
+def device_path_replay(inf, out0, N, A, B, K, S, cur, oracle_built, strategy="auto"):
     """Run the on-device search eagerly with every simulation's network outputs recorded, replay them through the CPU
-    oracle tree (bit-exact selections, sampled sets, visit counts, values, Q), then require graph replay == eager."""
+    oracle tree (bit-exact selections, sampled sets, visit counts, values, Q), then require graph replay == eager.
+    Returns the search output and the oracle's path length of every simulation and tree, (S, B)."""
     from mazero_b200.mcts_sampled import SampledMCTS
 
     cfg = MockConfig(N, A, S, K)
@@ -58,7 +59,7 @@ def device_path_replay(inf, out0, N, A, B, K, S, cur, oracle_built):
     legal[..., 1] = 1
 
     def run(graph, record):
-        mcts = SampledMCTS(cfg, np.random.RandomState(1), use_cuda_graph=graph)
+        mcts = SampledMCTS(cfg, np.random.RandomState(1), use_cuda_graph=graph, search_strategy=strategy)
         if record is not None:
             mcts.batch_search(inf, out0, cur, factor, N, legal, "cuda:0", add_noise=True)  # builds the plan
             plan = next(iter(mcts._plans.values()))
@@ -78,8 +79,10 @@ def device_path_replay(inf, out0, N, A, B, K, S, cur, oracle_built):
     orc = oracle_built.OracleTreeBatch(B, Nt, A, K, S, cfg.tree_value_stat_delta_lb, tree_seed, cfg.mcts_rho, cfg.mcts_lambda)
     orc.prepare(plan.root_r.cpu().numpy(), plan.root_v.cpu().numpy(), plan.root_p.cpu().numpy(), plan.root_b.cpu().numpy(),
                 K, cfg.root_exploration_fraction, plan.root_n.cpu().numpy())
+    lens = []
     for s, (rew, val, p, b, ix, act) in enumerate(rec):
         oix, _, oact = orc.batch_selection(cfg.pb_c_base, cfg.pb_c_init, cfg.discount)
+        lens.append(orc.stats()[1])
         assert np.array_equal(np.asarray(oix, np.int32), ix.cpu().numpy()), f"sim {s}: hidden_state_index_x"
         assert np.array_equal(oact, act.cpu().numpy()), f"sim {s}: selected actions"
         orc.batch_expansion_and_backup(s + 1, cfg.discount, K, rew.cpu().numpy(), val.cpu().numpy(), p.cpu().numpy(), b.cpu().numpy())
@@ -100,7 +103,7 @@ def device_path_replay(inf, out0, N, A, B, K, S, cur, oracle_built):
             assert np.array_equal(x, y), f
         else:
             assert x == y, f
-    return eager
+    return eager, np.stack(lens)
 
 
 @pytest.mark.parametrize("mode", ["bf16", "fp32"])

@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from _harness import MCTS, SHAPES, Inputs, assert_same, drive
+from _harness import MCTS, SHAPES, Inputs, assert_same, drive, drive_fused
 from test_oracle import GOLDEN, check_golden
 
 pytestmark = pytest.mark.gpu
@@ -67,6 +67,84 @@ def test_cuda_tree_long_rng_stream(cytree, oracle_built):
     ours = cytree.Tree_batch(B, N, A, K, S, 0.01, 1234567, 0.75, 0.8)
     orc = oracle_built.OracleTreeBatch(B, N, A, K, S, 0.01, 1234567, 0.75, 0.8, kind="port")
     assert_same(drive(ours, inp, K), drive(orc, inp, K), exact=True)
+
+
+# The fused step of the on-device loop (k_expand_backup_select2) holds the wide selection (tree_step.cuh: select_path_wide), taken
+# when the previous path had at least wide_min_len = 3 + 2 ceil((S+1)/32) nodes; MAZ_SELECT_WIDE=1 takes it at every selection
+# (except where the RNG words it needs straddle the end of the mt19937 block), =0 never.
+# name: (B, N, A, K, S, seed of the injected arrays, tree seed, what the oracle must show the case reaches)
+FUSED_CASES = {
+    **{f"{s}/{m}": (*SHAPES[s], 1, 4, ()) for s in SHAPES for m in ("random", "quantized")},
+    # K = 1 chains: the last path has S nodes (longer than a warp), the value log fills to within 8 entries of its capacity
+    "chain_s120": (3, 1, 2, 1, 120, 123, 41, ("deep", "chain")),
+    "chain_s200": (24, 3, 9, 1, 200, 224, 41, ("deep", "chain")),
+    "k2_s150": (16, 2, 6, 2, 150, 166, 41, ("wide",)),          # two children per node: the wide form's UCB choice matters
+    "long_rng": (8, 13, 7, 9, 60, 2, 1234567, ()),             # 2 K N = 234 draws per expansion
+    "slots": (2, 3, 6, 32, 2045, 2047, 41, ("slots",)),         # K (S+2) = 65504 node slots: slot indices above 32767
+    "wpb2": (lambda sms: 8 * sms + 317, 2, 5, 3, 12, 3, 41, ("wide",)),       # two trees per block, the last block ragged (1501 on a B200)
+    "wpb4": (lambda sms: 16 * sms + 133, 2, 5, 3, 12, 4, 41, ("wide",)),      # four trees per block, the last block ragged (2501 on a B200)
+}
+_FUSED_ORACLE = {}
+
+
+class _PathLog:
+    """A tree batch that records its per-tree path length (`stats()[1]`) after every selection."""
+
+    def __init__(self, tree):
+        self.tree, self.lens = tree, []
+
+    def __getattr__(self, name):
+        return getattr(self.tree, name)
+
+    def batch_selection(self, *a):
+        r = self.tree.batch_selection(*a)
+        self.lens.append(self.tree.stats()[1].copy())
+        return r
+
+
+def _fused_case(name, oracle_built):
+    import torch
+
+    B, N, A, K, S, seed, tree_seed, reach = FUSED_CASES[name]
+    if callable(B):
+        B = B(torch.cuda.get_device_properties(0).multi_processor_count)
+    mode = name.split("/")[1] if "/" in name else "random"
+    inp = Inputs(B, N, A, S, seed=seed, mode=mode, legal_frac=0.7 if "/" in name else None)
+    if name not in _FUSED_ORACLE:
+        orc = _PathLog(oracle_built.OracleTreeBatch(B, N, A, K, S, MCTS["delta_lb"], tree_seed, MCTS["rho"], MCTS["lam"], kind="port"))
+        want = drive(orc, inp, K)
+        lens = np.stack(orc.lens)                                       # (S, B)
+        tot = orc.stats()[0]
+        log_len = 1 + (lens + 1).sum(axis=0)                            # root entry + one entry per path level and simulation
+        wide_min_len = 3 + 2 * ((S + 1 + 31) // 32)
+        above = int((lens[:-1] >= wide_min_len).sum())                  # selections after which the next one is wide by default
+        print(f"{name}: B={B} largest path {lens.max()}, longest value log {log_len.max()} (capacity {1 + S * (S + 3) // 2 + 8}), "
+              f"selections at or above wide_min_len {wide_min_len}: {above}, most nodes {tot.max()}")
+        if "deep" in reach:
+            assert lens.max() > 32 and log_len.max() > 256
+        if "chain" in reach:
+            assert K == 1 and (lens[-1] == S).all() and (log_len == 1 + S * (S + 3) // 2).all()
+        if "deep" in reach or "wide" in reach:
+            assert above > 0
+        if "slots" in reach:
+            assert tot.max() > 32768
+        _FUSED_ORACLE[name] = want
+    return (B, N, A, K, S, tree_seed), inp, _FUSED_ORACLE[name]
+
+
+@pytest.mark.parametrize("select_wide", [None, "0", "1"], ids=["default", "wide0", "wide1"])
+@pytest.mark.parametrize("name", list(FUSED_CASES))
+def test_fused_step_matches_oracle(cytree, oracle_built, monkeypatch, name, select_wide):
+    """The on-device loop's launch order (prepare, selection, S-1 fused expansion + backup + selection, the last expansion +
+    backup, readouts) on injected arrays, bit for bit against the oracle, with the wide selection at its default threshold,
+    forced off and forced on."""
+    (B, N, A, K, S, tree_seed), inp, want = _fused_case(name, oracle_built)
+    if select_wide is None:
+        monkeypatch.delenv("MAZ_SELECT_WIDE", raising=False)
+    else:
+        monkeypatch.setenv("MAZ_SELECT_WIDE", select_wide)              # read by the tree layout when the batch is created
+    ours = cytree.Tree_batch(B, N, A, K, S, MCTS["delta_lb"], tree_seed, MCTS["rho"], MCTS["lam"])
+    assert_same(drive_fused(ours, inp, K), want, exact=True, what=f"{name}/{select_wide}: ")
 
 
 def test_root_index_offset_makes_shards_equal_to_the_whole(cytree):
@@ -131,6 +209,8 @@ def test_reset_reuses_arena(cytree):
 def test_errors_are_runtime_errors(cytree):
     with pytest.raises(RuntimeError):
         cytree.Tree_batch(4, 1, 3, 64, 5, 0.01, 0, 0.75, 0.8)  # K > 32
+    with pytest.raises(RuntimeError):
+        cytree.Tree_batch(2, 3, 6, 32, 2046, 0.01, 0, 0.75, 0.8)  # K (S+2) = 65536 node slots: more than 16-bit slots address
     t = cytree.Tree_batch(4, 1, 3, 2, 5, 0.01, 0, 0.75, 0.8)
     with pytest.raises(RuntimeError):
         t.batch_selection(19652.0, 1.25, 0.99)  # before prepare
